@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the judged harness (one JSON line on stdout, see the contract in DESIGN.md section 6).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload spike|tnc] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload spike|tnc] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of a hot path over one batch of synthetic input that is already resident in HBM
 (`value`), or that starts in pinned host memory and ends with the results back on the host (`e2e`).
@@ -40,6 +40,19 @@ assert sum(GRCH38) == 3088269832
 
 def log(*a):
     print(*a, file=sys.stderr, flush=True)
+
+
+def dump(args, D, name, arr, dtype=None, replicated=False):
+    """--dump-outputs: writes one output of the timed path as DIR/<name>.npy (float64 unless `dtype` says float32), so that two builds
+    can be compared output for output on the same seeded input.  When several ranks run, an output every rank holds alike
+    (`replicated`) is written by rank 0 alone; any other goes to DIR/<name>.rank<r>.npy."""
+    import numpy as np
+    if not args.dump_outputs or (replicated and D.rank != 0):
+        return
+    os.makedirs(args.dump_outputs, exist_ok=True)
+    if D.on and not replicated:
+        name = "%s.rank%d" % (name, D.rank)
+    np.save(os.path.join(args.dump_outputs, name + ".npy"), np.asarray(arr, dtype=dtype or np.float64))
 
 
 def measured_peaks():
@@ -271,6 +284,7 @@ def run_tnc(args, D, ctx=None):
     fix_ms, fix_n = ctx.profile_read(1)
     ms = D.max(ms)
     counts = d_counts.cpu().numpy().copy()                                 # after the all-reduce: the whole file's counts on every rank
+    dump(args, D, "tnc_counts", counts, replicated=True)
 
     # the sharded counts must equal the one-GPU counts of the whole file (rank 0 checks, outside the timed region)
     if D.on and D.rank == 0:
@@ -280,7 +294,7 @@ def run_tnc(args, D, ctx=None):
         assert np.array_equal(d_whole.cpu().numpy(), counts), "sharded TNC counts differ from the single-GPU counts"
 
     # ---- e2e: host buffers through ssb_tnc_count_host (H2D inside the timed region, counts back on the host, all-reduce included)
-    e2e_steps = max(1, min(args.steps, 5))
+    e2e_steps = args.steps
     hp = ctx.host_alloc(max(n, 1))
     ctx.d2h(hp, piece.data_ptr(), n)
     ctx.sync()
@@ -414,7 +428,12 @@ def main():
     ap.add_argument("--scale", type=float, default=1.0, help="shrink the workload (development only; the judged run uses 1.0)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-tnc", action="store_true", help="spike workload only (development)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     # only the JSON line may reach stdout: libraries (NCCL prints its version there) go to stderr meanwhile
     sys.stdout.flush()
@@ -464,9 +483,7 @@ def main():
         res, ctx = bench_spike.run(args, D)
         # the other hot path rides in the same line (BASELINE's metric names both)
         if not args.no_tnc:
-            tnc_args = argparse.Namespace(**vars(args))
-            tnc_args.steps = max(args.steps, 10)
-            tnc, counts = run_tnc(tnc_args, D, ctx)
+            tnc, counts = run_tnc(args, D, ctx)
             if D.rank == 0 and not args.no_cpu_baseline:
                 tnc["cpu_baseline"] = tnc_parity_baseline(ctx)
             res["tnc"] = tnc

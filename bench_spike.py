@@ -162,6 +162,54 @@ def traffic_from_profile(scale):
         return None, None
 
 
+DUMP_BLOCK = 1 << 16                   # bytes of spiked SAM per entry of spike_sam_block_sums (on one rank)
+DUMP_WINDOWS, DUMP_WINDOW = 64, 1 << 16
+# the Stats fields that are results of the pass (the counters of the reference's stats block, the rand() draws); timings and
+# scheduling counters (chain chunks, streamed pieces, window retries) may differ between builds that compute the same thing
+DUMP_STATS = ("alignmentCount", "numberOfLociCovered", "totalFoldCoverage", "maxDepth", "n_lines", "n_kept", "in_bytes", "out_bytes",
+              "n_hits", "rng_draws", "rng_k_in", "rng_k_out")
+
+
+def dump_spike(args, D, ctx, d_out, out_bytes, res, n_targets, st):
+    """--dump-outputs for one spike pass: what a caller of ssb_spike_run[_shard]_device receives.  The spiked SAM body is too large to
+    store, so it goes as the byte sum of every block (the whole body) plus windows of 64 KiB at seeded offsets, byte for byte; the
+    targets go as one row per target this rank owns (target index first).  On N ranks the blocks are N x 64 KiB long and each rank
+    writes 64 / N windows, so the files of all ranks together stay near the size of one rank's at N = 1 (about 19 MB at C2)."""
+    if not args.dump_outputs:
+        return
+    from bench import dump
+    from stochasticsim_b200 import spike as sp
+    block = DUMP_BLOCK * D.world
+    chunk = block * max(1, (1 << 28) // block)
+    buf = np.empty(chunk, dtype=np.uint8)
+    sums = []
+    for c0 in range(0, out_bytes, chunk):
+        m = min(chunk, out_bytes - c0)
+        ctx.d2h(buf.ctypes.data, d_out + c0, m)
+        ctx.sync()
+        full = m // block * block
+        sums.append(buf[:full].reshape(-1, block).sum(axis=1, dtype=np.uint64))
+        if full < m:
+            sums.append(buf[full:m].sum(dtype=np.uint64, keepdims=True))
+    dump(args, D, "spike_sam_block_sums", np.concatenate(sums) if sums else np.zeros(0))
+    w, nw = min(DUMP_WINDOW, out_bytes), max(1, DUMP_WINDOWS // D.world)
+    offs = np.sort(np.random.default_rng(434).integers(0, out_bytes - w + 1, size=nw))
+    win = np.empty((nw, w), dtype=np.uint8)
+    for i, o in enumerate(offs):
+        ctx.d2h(win[i].ctypes.data, d_out + int(o), w)
+    ctx.sync()
+    dump(args, D, "spike_sam_window_offsets", offs)
+    dump(args, D, "spike_sam_windows", win, np.float32)
+    tr = []
+    for i in range(n_targets):
+        r = res[i]
+        if r.status != sp.T_ELSEWHERE:
+            tr.append([i, r.status, r.at_tid, r.at_pos, r.locus_index, r.ref_base, r.mutant_allele, r.filter, r.ref_cnt, r.mut_cnt,
+                       *r.err_cnt, r.rng_offset])
+    dump(args, D, "spike_targets", np.array(tr, dtype=np.float64).reshape(len(tr), 15))
+    dump(args, D, "spike_stats", [getattr(st, k) for k in DUMP_STATS])
+
+
 def run(args, D):
     import torch
     import stochasticsim_b200 as ssb
@@ -274,9 +322,10 @@ def run(args, D):
         for a, b in zip(chain, chain[1:]):
             assert int(a[1]) == int(b[0]), "rand() offset hand-off broken: %r" % (chain,)
         assert int(chain[0][0]) == 0
+    dump_spike(args, D, ctx, d_out, out_bytes, res, len(targets), st)
 
     # ---- e2e: pinned host SAM body in, spiked SAM body back on the host
-    e2e_steps = max(1, min(args.steps, 3))
+    e2e_steps = args.steps
     outn = C.c_size_t()
     Lb = sp._bind()
 
@@ -539,7 +588,7 @@ def run_panel(args, D):
     tarr = S.make_targets(targets)
     res = (sp.TargetResult * len(targets))()
     st = sp.Stats()
-    steps, warm = max(1, min(args.steps, 5)), 1
+    steps, warm = args.steps, 1
     for _ in range(warm):
         out_bytes = S.run_device(d_in, n, d_out, n + 1, tarr, len(targets), SPIKE_SEED, res, st)
     ctx.sync()
@@ -553,6 +602,7 @@ def run_panel(args, D):
                     stage_ms[k] = stage_ms.get(k, 0.0) + v
         ms = ctx.timer_stop()
     stats = st.as_dict()
+    dump_spike(args, D, ctx, d_out, out_bytes, res, len(targets), st)
     entries = sum(r.ref_cnt + r.mut_cnt + sum(r.err_cnt) for r in res if r.status == sp.T_HIT)
     ms_step = ms / steps
     out = {

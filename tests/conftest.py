@@ -29,8 +29,10 @@ def built():
 
 @pytest.fixture(scope="session")
 def ref_dir():
-    """oracle/_ref/: the UNMODIFIED reference compiled here (travels to the GPU box as binaries); None if absent."""
+    """oracle/_ref/: the UNMODIFIED reference, compiled from the upstream stochasticSim sources that STOCHASTICSIM_SRC points to
+    (they are not part of this repository); None if absent."""
     d = os.path.join(ROOT, "oracle", "_ref")
-    if os.path.exists("/root/reference/tncCountsProfile.c") and not os.path.exists(os.path.join(d, "stochasticSpike")):
-        _make("ref")
+    src = os.environ.get("STOCHASTICSIM_SRC", "")
+    if src and os.path.exists(os.path.join(src, "tncCountsProfile.c")) and not os.path.exists(os.path.join(d, "stochasticSpike")):
+        _make("ref", "REFERENCE=" + os.path.abspath(src))
     return d if os.path.exists(os.path.join(d, "tncCountsProfile")) else None

@@ -2,9 +2,10 @@
 
  * against oracle/_ref/stochasticSpike = the UNMODIFIED reference source compiled over oracle/shim/ (only the
    htslib I/O + pileup layer is restated there; "reference logic over shimmed htslib"), byte for byte on SAM,
-   truth.vcf and stdout;
+   truth.vcf and stdout -- or, where that binary is not built, against the digests of its answers on the same inputs
+   (tests/golden/reference_digests.json);
  * against the committed golden fixture tests/golden/spike_toy/ (made by tests/golden/make_spike_golden.py with
-   that same reference binary), which also travels to the GPU box where /root/reference does not exist;
+   that same reference binary), which needs no reference binary;
  * against the glibc rand() known answers of SURVEY.md App. C."""
 import os
 
@@ -12,23 +13,48 @@ import numpy as np
 import pytest
 
 import oracle_bind as ob
+import reference_digests as rd
 import spike_cases as sc
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLD = os.path.join(HERE, "golden", "spike_toy")
 
 
+def _matches_reference(key, prefix, seed, tmp_path, ref_dir):
+    """The restatement against the reference over the shim on one input: byte for byte against oracle/_ref/stochasticSpike when it
+    is built, else against the digests of that binary's answers in tests/golden/reference_digests.json."""
+    b = sc.run_cli(sc.ORACLE, prefix, str(tmp_path / "ora"), seed=seed, cmdname="stochasticSpike")
+    if ref_dir is not None and os.path.exists(sc.REF):
+        a = sc.run_cli(sc.REF, prefix, str(tmp_path / "ref"), seed=seed)
+        assert a[0] == b[0] == 0
+        assert a[2] == b[2], "SAM differs"
+        assert a[3] == b[3], "truth.vcf differs"
+        assert a[1] == b[1], "stdout differs"
+        return
+    gold = rd.load()["spike"][key]
+    assert gold["seed"] == seed
+    assert rd.spike_inputs(prefix) == gold["inputs"], "the generator no longer makes the input the digests were recorded on"
+    got = rd.spike_outputs(b, prefix)
+    assert got["rc"] == gold["outputs"]["rc"] == 0
+    assert got["out.sam"] == gold["outputs"]["out.sam"], "SAM differs"
+    assert got["truth.vcf"] == gold["outputs"]["truth.vcf"], "truth.vcf differs"
+    assert got["stdout"] == gold["outputs"]["stdout"], "stdout differs"
+
+
+def reference_case(family, name, outdir):
+    """(input prefix, seed) of one input of the two parametrized tests below."""
+    if family == "shim":
+        return sc.generate(name, outdir), 434
+    if name in LONG_READS:
+        from test_spike_gpu import _long_read_case
+        return _long_read_case(outdir, LONG_READS[name]), 435
+    return sc.generate("plain", outdir, **EXTRA_CASES[name]), 435
+
+
 @pytest.mark.parametrize("name", sorted(sc.CASES))
 def test_restatement_matches_reference_over_shim(name, tmp_path, ref_dir):
-    if ref_dir is None or not os.path.exists(sc.REF):
-        pytest.skip("oracle/_ref not built (reference sources not present on this box)")
-    prefix = sc.generate(name, str(tmp_path))
-    a = sc.run_cli(sc.REF, prefix, str(tmp_path / "ref"))
-    b = sc.run_cli(sc.ORACLE, prefix, str(tmp_path / "ora"), cmdname="stochasticSpike")
-    assert a[0] == b[0] == 0
-    assert a[2] == b[2], "SAM differs"
-    assert a[3] == b[3], "truth.vcf differs"
-    assert a[1] == b[1], "stdout differs"
+    prefix, seed = reference_case("shim", name, str(tmp_path))
+    _matches_reference("shim/" + name, prefix, seed, tmp_path, ref_dir)
 
 
 def _gold(name):
@@ -91,16 +117,5 @@ LONG_READS = {"long5k": [5000] * 150, "long_mix": [40000] * 12 + [5000] * 40 + [
 def test_restatement_matches_reference_on_gpu_test_inputs(name, tmp_path, ref_dir):
     """Every input family the GPU parity tests use beyond spike_cases.CASES: the restatement must agree with the unmodified
     reference over the shim there too, or those GPU tests would pin nothing."""
-    if ref_dir is None or not os.path.exists(sc.REF):
-        pytest.skip("oracle/_ref not built (reference sources not present on this box)")
-    if name in LONG_READS:
-        from test_spike_gpu import _long_read_case
-        prefix = _long_read_case(str(tmp_path), LONG_READS[name])
-    else:
-        prefix = sc.generate("plain", str(tmp_path), **EXTRA_CASES[name])
-    a = sc.run_cli(sc.REF, prefix, str(tmp_path / "ref"), seed=435)
-    b = sc.run_cli(sc.ORACLE, prefix, str(tmp_path / "ora"), seed=435, cmdname="stochasticSpike")
-    assert a[0] == b[0] == 0
-    assert a[2] == b[2], "SAM differs"
-    assert a[3] == b[3], "truth.vcf differs"
-    assert a[1] == b[1], "stdout differs"
+    prefix, seed = reference_case("gpu_inputs", name, str(tmp_path))
+    _matches_reference("gpu_inputs/" + name, prefix, seed, tmp_path, ref_dir)

@@ -9,6 +9,7 @@ import pytest
 
 import fasta_cases as fc
 import oracle_bind as ob
+import reference_digests as rd
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 
@@ -51,16 +52,21 @@ def test_nul_rejected():
 
 
 def test_fuzz_against_compiled_reference(ref_dir, tmp_path):
-    if ref_dir is None:
-        pytest.skip("oracle/_ref not built (reference sources not present on this box)")
-    rng = random.Random(11)
-    exe = os.path.join(ref_dir, "tncCountsProfile")
-    for i in range(300):
-        data = fc.random_fasta(rng) if i >= len(fc.EDGE) else fc.EDGE[i]
+    """Against oracle/_ref/tncCountsProfile when it is built, else against the digests of its stdout on the same inputs
+    (tests/golden/reference_digests.json)."""
+    gold = rd.load()["tnc_fuzz"] if ref_dir is None else None
+    inputs = rd.tnc_fuzz_inputs()
+    assert gold is None or len(gold) == len(inputs)
+    for i, data in enumerate(inputs):
+        got = ob.tnc_text(ob.tnc_counts(data))
+        if gold is not None:
+            assert [len(data), rd.sha(data)] == gold[i][:2], "input %d is not the one the digest was recorded on" % i
+            assert rd.sha(got.encode()) == gold[i][2], data
+            continue
         p = tmp_path / "f.fa"
         p.write_bytes(data)
-        ref = subprocess.run([exe, str(p)], capture_output=True).stdout.decode()
-        assert ob.tnc_text(ob.tnc_counts(data)) == ref, data
+        ref = subprocess.run([os.path.join(ref_dir, "tncCountsProfile"), str(p)], capture_output=True).stdout.decode()
+        assert got == ref, data
 
 
 def test_missing_file_exit_status(ref_dir):
