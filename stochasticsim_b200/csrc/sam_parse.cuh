@@ -766,8 +766,9 @@ __device__ __forceinline__ uint32_t long_fields(const uint8_t *L, uint32_t seq_o
             if (CMP) {
                 const uint32_t q = 4 * j + k - sh;
                 uint32_t rb = (rf >> (8 * k)) & 0xffu;
-                if (rb == 0xffu) rb = ref_raw[q];                          // not A/C/G/T/N: the tally compares with the byte as it is
-                if (sb != rb || qb == '!') {
+                if (rb == 0xffu) rb = ref_raw[q];                          // not A/C/G/T: the tally compares with the byte as it is
+                // a read N is never a reference base, not even over a reference N (reads through the N runs of a real reference)
+                if (sb != rb || qb == '!' || sb == 'N') {
                     const unsigned int slot = atomicAdd(s_nexc, 1u);
                     if (slot < (unsigned int)EXC_BUF) excbuf[slot] = (line_in_tile << 16) | q;
                     else bad |= 2u;
@@ -1130,7 +1131,8 @@ parse_kernel(const uint8_t *__restrict__ body, size_t n, ContigNames names, SamR
                 const int nwords = ((w_hi - w_lo + 3) >> 2) + 1;
                 for (int w = tid_; w < nwords; w += THREADS) {
                     const uint32_t x = __funnelshift_r(__ldg(rw + w), __ldg(rw + w + 1), ra * 8);
-                    dw[w] = x | ((non_acgtn_bytes(x) >> 7) * 0xffu);           // anything but A C G T N can never equal a valid SEQ byte
+                    // anything but A C G T can never equal a valid SEQ byte; N too, so that a read over a reference N is always looked at
+                    dw[w] = x | (((non_acgtn_bytes(x) | zero_bytes(x ^ 0x4E4E4E4Eu)) >> 7) * 0xffu);
                 }
                 in_win = elig && gi < rec_cap && gi < (1ull << 47) && r.tid == wtid && r.pos >= w_lo && r.end <= w_lo + REFW;
             } else wtid = -1;

@@ -834,7 +834,8 @@ __device__ __forceinline__ uint32_t exc_word(const uint8_t *seq, const uint8_t *
 {
     const uint32_t sq = ldg_u32_unaligned(seq + w);
     const uint32_t ql = qstar ? 0x7e7e7e7eu : ldg_u32_unaligned(qual + w);
-    return (~samparse::zero_bytes(sq ^ refw) | samparse::zero_bytes(ql ^ 0x21212121u)) & 0x80808080u;
+    // a read N counts nothing, also where it equals a reference N (reads through the N runs of a real reference)
+    return (~samparse::zero_bytes(sq ^ refw) | samparse::zero_bytes(sq ^ 0x4E4E4E4Eu) | samparse::zero_bytes(ql ^ 0x21212121u)) & 0x80808080u;
 }
 
 // the rare path of the fast tally: one exceptional base of read o at reference position x, evaluated exactly
@@ -954,7 +955,7 @@ tally_resolve_kernel(TallyArgs A, const unsigned long long *__restrict__ list, u
         uint8_t b; int bq; bool sk;
         base_at(cov[m], x, b, bq, sk);
         // a plain base of a list-settled neighbour has no entry of its own: it matters only if it was marked handled here
-        if (b == F && bq != 0 && tally_is_listed(A, cord[m], A.recs[A.k_rec[cord[m]]], n_odd, bloom)) tally_add(A, g, chain_contribution(cov, nc, m, x, F));
+        if (b == F && b != 'N' && bq != 0 && tally_is_listed(A, cord[m], A.recs[A.k_rec[cord[m]]], n_odd, bloom)) tally_add(A, g, chain_contribution(cov, nc, m, x, F));
     }
 }
 
