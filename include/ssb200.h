@@ -128,6 +128,7 @@ int ssb_tnc_allreduce(ssb_ctx *ctx, void *nccl_comm, int64_t *d_counts64);
  * counts of a partition of [0, n_intervals) add up to the whole (one range per GPU, then ssb_tnc_allreduce). */
 typedef struct ssb_fasta_contig { uint64_t seq_off; int64_t len; uint32_t line_bases, line_bytes; } ssb_fasta_contig;
 typedef struct ssb_bed_interval { int32_t contig, reserved; int64_t start, end; } ssb_bed_interval;      /* 0-based, half open */
+/* SSB_E_FORMAT when a record's sequence lines are not all as wide as its first one (only the last may be shorter). */
 int ssb_fasta_index(const uint8_t *fasta, size_t n, ssb_fasta_contig *out, const char **names, uint32_t *name_lens, size_t cap, size_t *n_out);
 int ssb_tnc_count_bed_device(ssb_ctx *ctx, const uint8_t *d_fasta, size_t n, const ssb_fasta_contig *contigs, size_t n_contigs,
                              const ssb_bed_interval *intervals, size_t n_intervals, size_t first, size_t last, int64_t *d_counts64);

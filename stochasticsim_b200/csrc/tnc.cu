@@ -776,8 +776,9 @@ extern "C" int ssb_tnc_count_bed_device(ssb_ctx *ctx, const uint8_t *d_fasta, si
 }
 
 // .fai-style index of a FASTA text (host): one entry per '>' record, in file order.  names[i] points into the text (not NUL
-// terminated).  Like faidx it takes the line geometry from a record's first sequence line and expects every line but the last to
-// have that width ('>' cannot occur inside a sequence line, so the next record is found by a byte search, not line by line).
+// terminated).  Like faidx it takes the line geometry from a record's first sequence line and refuses (SSB_E_FORMAT) a record
+// in which another line but the last has a different width; blank lines after the last sequence line are allowed ('>' cannot
+// occur inside a sequence line, so the next record is found by a byte search, not line by line).
 extern "C" int ssb_fasta_index(const uint8_t *fa, size_t n, ssb_fasta_contig *out, const char **names, uint32_t *name_lens, size_t cap, size_t *n_out)
 {
     if ((!fa && n) || !n_out) return SSB_E_ARG;
@@ -800,25 +801,33 @@ extern "C" int ssb_fasta_index(const uint8_t *fa, size_t n, ssb_fasta_contig *ou
             if (gp == s0 || fa[gp - 1] == '\n') { end = gp; break; }
             r = gp + 1;
         }
+        ssb_fasta_contig c; c.seq_off = s0; c.len = 0; c.line_bases = 0; c.line_bytes = 0;
+        const size_t bytes = end - s0;
+        if (bytes) {
+            const uint8_t *nl2 = (const uint8_t *)memchr(fa + s0, '\n', bytes);
+            const size_t l_bytes = nl2 ? (size_t)(nl2 - (fa + s0)) + 1 : bytes;            // first line incl. its newline
+            size_t term = nl2 ? 1 : 0; if (nl2 && l_bytes >= 2 && fa[s0 + l_bytes - 2] == '\r') term = 2;
+            c.line_bytes = (uint32_t)l_bytes; c.line_bases = (uint32_t)(l_bytes - term);
+            if (c.line_bases) {
+                // up to the last byte that is not a line terminator: blank lines after the last sequence line hold no base
+                size_t t = bytes;
+                while (t && (fa[s0 + t - 1] == '\n' || fa[s0 + t - 1] == '\r')) t--;
+                const size_t full = term ? t / l_bytes : 0, rest = term ? t % l_bytes : t;      // (term 0: one unterminated line)
+                // every line but the last ends where the first one does, with the same terminator, and the last is no longer: any
+                // other record (a blank line inside it, a ragged line) would put bases where the geometry does not look for them
+                bool uniform = rest <= c.line_bases && !memchr(fa + s0 + full * l_bytes, '\n', rest);
+                for (size_t j = 1; uniform && j <= full; j++) {
+                    const uint8_t *x = fa + s0 + j * l_bytes;
+                    uniform = x[-1] == '\n' && (x[-2] == '\r') == (term == 2);
+                }
+                if (!uniform) return SSB_E_FORMAT;
+                c.len = (int64_t)(full * c.line_bases + rest);
+            }
+        }
         if (k < cap && out) {
             size_t q = p + 1; while (q < e && fa[q] != ' ' && fa[q] != '\t' && fa[q] != '\r') q++;
             if (names) names[k] = (const char *)fa + p + 1;
             if (name_lens) name_lens[k] = (uint32_t)(q - p - 1);
-            ssb_fasta_contig c; c.seq_off = s0; c.len = 0; c.line_bases = 0; c.line_bytes = 0;
-            const size_t bytes = end - s0;
-            if (bytes) {
-                const uint8_t *nl2 = (const uint8_t *)memchr(fa + s0, '\n', bytes);
-                const size_t l_bytes = nl2 ? (size_t)(nl2 - (fa + s0)) + 1 : bytes;            // first line incl. its newline
-                size_t term = nl2 ? 1 : 0; if (nl2 && l_bytes >= 2 && fa[s0 + l_bytes - 2] == '\r') term = 2;
-                c.line_bytes = (uint32_t)l_bytes; c.line_bases = (uint32_t)(l_bytes - term);
-                if (c.line_bases) {
-                    const size_t full = bytes / l_bytes, rest = bytes % l_bytes;
-                    size_t tail = rest;                       // a last, shorter line (with or without terminator)
-                    if (tail && fa[s0 + bytes - 1] == '\n') tail--;
-                    if (tail && term == 2 && fa[s0 + full * l_bytes + tail - 1] == '\r') tail--;
-                    c.len = (int64_t)(full * c.line_bases + tail);
-                }
-            }
             out[k] = c;
         }
         k++;

@@ -119,7 +119,8 @@ int main(int argc, char **argv)
     /* BED mode (second argument) */
     ssb_fasta_contig *contigs = NULL; ssb_bed_interval *iv = NULL; size_t n_contigs = 0, n_iv = 0;
     if (argc > 2 && argv[2]) {
-        ssb_fasta_index(data, n, NULL, NULL, NULL, 0, &n_contigs);
+        int rc = ssb_fasta_index(data, n, NULL, NULL, NULL, 0, &n_contigs);
+        if (rc) { fprintf(stderr, "tncCountsProfile: %s: a record's lines are not all as wide as its first one (%s)\n", argv[1], ssb_strerror(rc)); return 3; }
         contigs = malloc((n_contigs + 1) * sizeof *contigs);
         const char **names = malloc((n_contigs + 1) * sizeof *names); uint32_t *nlens = malloc((n_contigs + 1) * sizeof *nlens);
         ssb_fasta_index(data, n, contigs, names, nlens, n_contigs, &n_contigs);

@@ -1,6 +1,8 @@
 """Seeded FASTA inputs shared by the oracle tests (CPU) and the parity tests (GPU)."""
 import random
 
+import numpy as np
+
 # SURVEY.md App. B known answers: produced by running the reference's own compiled binary.
 KAT = [
     (b">c1\nACGT\nGGCC\n", {"ACG": 2, "CCA": 1, "GCC": 2}),
@@ -57,3 +59,24 @@ def genome_like(rng: random.Random, n_bases: int, width=60, n_block=None, lower_
         for i in range(0, per, width):
             out.append(bytes(seq[i:i + width]) + b"\n")
     return b"".join(out)
+
+
+def shard_counts_with_carry(data: bytes, lo: int, hi: int):
+    """Counts of data[lo:hi] given everything before lo, via the oracle: counts(data[:hi]) - counts(data[:lo]) is NOT
+    what a rank can compute, so emulate the device contract instead: prepend the minimal context the carried state
+    stands for and subtract its own windows."""
+    import oracle_bind as ob
+    import stochasticsim_b200 as ssb
+    st = ssb.tnc.carry_after(np.frombuffer(data, dtype=np.uint8)[:lo]) if lo else None
+    piece = data[lo:hi]
+    if st is None:
+        return ob.tnc_counts(piece)
+    # context equivalent to the state: the carried last byte of the nearest kept line, then the fragment of the current line
+    started, prev, carry, frag_nonempty, frag_first, frag_has_base = st.as_tuple()
+    ctx = b""
+    if carry:
+        ctx += b"A" + bytes([carry]) + b"\n"          # a kept line ending in `carry` ("A" makes it kept, adds no window by itself)
+    j = data.rfind(b"\n", 0, lo) + 1                     # the current line's fragment before the cut, verbatim
+    frag = data[j:lo]
+    base = ob.tnc_counts(ctx + frag) if (ctx or frag) else np.zeros(64, dtype=np.int64)
+    return ob.tnc_counts(ctx + frag + piece) - base

@@ -17,34 +17,14 @@ sys.path.insert(0, HERE)
 sys.path.insert(0, os.path.dirname(HERE))
 
 
-def _shard_counts_with_carry(data: bytes, lo: int, hi: int):
-    """Counts of data[lo:hi] given everything before lo, via the oracle: counts(data[:hi]) - counts(data[:lo]) is NOT
-    what a rank can compute, so emulate the device contract instead: prepend the minimal context the carried state
-    stands for and subtract its own windows."""
-    import oracle_bind as ob
-    import stochasticsim_b200 as ssb
-    st = ssb.tnc.carry_after(data[:lo]) if lo else None
-    piece = data[lo:hi]
-    if st is None:
-        return ob.tnc_counts(piece)
-    # context equivalent to the state: the carried last byte of the nearest kept line, then the fragment of the current line
-    started, prev, carry, frag_nonempty, frag_first, frag_has_base = st.as_tuple()
-    ctx = b""
-    if carry:
-        ctx += b"A" + bytes([carry]) + b"\n"          # a kept line ending in `carry` ("A" makes it kept, adds no window by itself)
-    j = data.rfind(b"\n", 0, lo) + 1                     # the current line's fragment before the cut, verbatim
-    frag = data[j:lo]
-    base = ob.tnc_counts(ctx + frag) if (ctx or frag) else np.zeros(64, dtype=np.int64)
-    return ob.tnc_counts(ctx + frag + piece) - base
-
-
 def _worker(rank, world, port, data, out_q):
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)
     dist.init_process_group("gloo", rank=rank, world_size=world)
     n = len(data)
     lo, hi = (n * rank // world) & ~31, n if rank == world - 1 else (n * (rank + 1) // world) & ~31
-    c = torch.from_numpy(_shard_counts_with_carry(data, lo, hi).astype(np.int64))
+    import fasta_cases as fc
+    c = torch.from_numpy(fc.shard_counts_with_carry(data, lo, hi).astype(np.int64))
     dist.all_reduce(c)                                   # the path's only collective: 64 int64 counters
     if rank == 0:
         out_q.put(c.numpy().tolist())
