@@ -14,6 +14,9 @@
 //   4. warps 1..3 parse the heads (QNAME .. TLEN) of one line per thread, lanes kept together (parse_head_conv);
 //   5. all threads stage the reference window under the tile's reads; warps 1..3 then check SEQ, QUAL and the reference
 //      in one pass (long_fields), list the exceptional bases and write the 64-byte SamRecs.
+// Two line parsers: the fast one of steps 4-5 (parse_head_conv + long_fields) for lines of the common shape, and the careful
+// parse_line() for the lines the fast one objects to, the lines beyond the first 96 of a tile, and the lines that end past the
+// staged window (those it reads from global memory).  They share the read filter (read_bam_filter) and the CIGAR ops (cigar_op).
 // Shared-memory regions change hands inside a tile (newline masks -> reference window, line starts -> exception buffer).
 // HBM traffic: the text is read once; 64 B per line and 8 B per exceptional base are written.
 #pragma once
@@ -71,6 +74,17 @@ __device__ __forceinline__ void shard_keep(SamRec &r, const ContigNames &names)
     if ((r.bits & REC_KEEP) && ((((unsigned long long)(uint32_t)r.tid << 32) | (uint32_t)r.end) - 1 < names.keep_lo)) r.bits &= (uint8_t)~REC_KEEP;
 }
 
+// The end of every line: a refused line (rc != 0) leaves an empty record and, if it is the first error, its code and offset;
+// the shard's lower bound applies; the record and its keys go to line g.
+__device__ __forceinline__ void store_line(SamRec &r, int rc, size_t s, unsigned long long g, const ContigNames &names,
+                                           SamRec *__restrict__ recs, size_t rec_cap, SpikeErr *__restrict__ err)
+{
+    if (rc) { if (atomicCAS(&err->code, 0, rc) == 0) err->where = s; memset(&r, 0, sizeof r); r.line_off = s; r.tid = -1; }
+    shard_keep(r, names);
+    if (g < rec_cap) { recs[g] = r; line_keys(names, g, r); }
+    else if (atomicCAS(&err->code, 0, SSB_E_NOMEM) == 0) err->where = s;
+}
+
 __device__ __forceinline__ uint32_t nl_mask16(uint4 v)
 {
     // 16-bit mask of '\n' bytes in 16 bytes
@@ -86,10 +100,25 @@ __device__ __forceinline__ uint32_t nl_mask16(uint4 v)
     return m;
 }
 
-struct Cursor {               // byte access: shared memory while inside the staged window, else global
-    const uint8_t *smem; const uint8_t *g; size_t base; size_t lim; size_t n;
-    __device__ __forceinline__ uint8_t at(size_t p) const { return p < lim ? smem[p - base] : (p < n ? g[p] : (uint8_t)'\n'); }
-};
+// read_bam (stochasticSpike.c:253-263) + bam_plp_push's tid test, on a parsed record
+__device__ __forceinline__ void read_bam_filter(SamRec &r)
+{
+    const bool pass = !(r.flag & (4 | 256 | 512 | 1024)) && r.mapq >= 30 && !((r.flag & 1) && !(r.flag & 2));
+    if (pass && r.tid >= 0) r.bits |= (r.end > r.pos) ? (REC_PUSHED | REC_KEEP) : REC_PUSHED;
+}
+
+// The class of a CIGAR op byte, branch free: CIG_OK for the nine ops (MIDNSHP=X), CIG_REF if it consumes the reference,
+// CIG_QRY if it consumes the query, CIG_M for M, = and X.  0 for any other byte.
+constexpr uint32_t CIG_REF = 1, CIG_QRY = 2, CIG_M = 4, CIG_OK = 8;
+__host__ __device__ constexpr uint32_t cig_bit(char op) { return 1u << (op - '='); }      // one bit per byte '=' .. 'X'
+__device__ __forceinline__ uint32_t cigar_op(uint32_t c)
+{
+    constexpr uint32_t M = cig_bit('M') | cig_bit('=') | cig_bit('X');
+    constexpr uint32_t REF = M | cig_bit('D') | cig_bit('N'), QRY = M | cig_bit('I') | cig_bit('S');
+    constexpr uint32_t OK = REF | QRY | cig_bit('H') | cig_bit('P');
+    const uint32_t i = c - '=', b = i <= (uint32_t)('X' - '=') ? 1u << i : 0u;
+    return ((b & REF) ? CIG_REF : 0u) | ((b & QRY) ? CIG_QRY : 0u) | ((b & M) ? CIG_M : 0u) | ((b & OK) ? CIG_OK : 0u);
+}
 
 __device__ __forceinline__ bool seq_char_ok(uint8_t c)
 {
@@ -99,32 +128,13 @@ __device__ __forceinline__ bool seq_char_ok(uint8_t c)
     return ((0x16e34cfu >> (c - 'A')) & 1u) != 0;          // A B C D G H K M N R S T V W Y
 }
 
-// Canonical decimal field ending at '\t' (what htslib prints back): digits only, no leading zero
-// unless the value is 0, value <= maxv.  On success p sits on the terminating tab.
-__device__ __forceinline__ int parse_udec(const Cursor &cur, size_t &p, size_t e, uint64_t maxv, uint64_t &out)
-{
-    size_t p0 = p; uint64_t v = 0;
-    while (p < e) {
-        uint8_t c = cur.at(p);
-        if (c == '\t') break;
-        if (c < '0' || c > '9') return SSB_E_FORMAT;
-        v = v * 10 + (c - '0');
-        if (v > maxv) return SSB_E_FORMAT;
-        p++;
-    }
-    if (p >= e || p == p0) return SSB_E_FORMAT;
-    if (p - p0 > 1 && cur.at(p0) == '0') return SSB_E_FORMAT;
-    out = v;
-    return 0;
-}
-
-// RNAME / RNEXT lookup: index of the first @SQ with that name, -1 if none
-__device__ __forceinline__ int name_lookup(const Cursor &cur, size_t p0, size_t len, const ContigNames &names, int hint)
+// RNAME / RNEXT lookup: index of the first @SQ named by the len bytes at p, -1 if none
+__device__ __forceinline__ int name_lookup(const uint8_t *p, uint32_t len, const ContigNames &names, int hint)
 {
     auto same = [&](int c) {
         uint32_t a = names.off[c], b = names.off[c + 1];
         if (b - a != len) return false;
-        for (size_t i = 0; i < len; i++) if ((uint8_t)names.text[a + i] != cur.at(p0 + i)) return false;
+        for (uint32_t i = 0; i < len; i++) if ((uint8_t)names.text[a + i] != p[i]) return false;
         return true;
     };
     if (hint >= 0 && hint < names.n && same(hint)) {
@@ -236,26 +246,14 @@ __host__ __device__ int aux_float_ok_t(const AT &at, size_t p, size_t q)
     return 0;
 }
 
-__device__ int aux_ok(const Cursor &cur, size_t p, size_t q)
-{
-    return aux_ok_t([&](size_t i) -> uint8_t { return cur.at(i); }, p, q);
-}
-// the same for a line that lies in the staged window: L = first byte of the line, offsets relative to it
-__device__ int aux_ok_smem(const uint8_t *L, uint32_t p, uint32_t q)
+// L = first byte of the line, offsets relative to it
+__device__ int aux_ok(const uint8_t *L, uint32_t p, uint32_t q)
 {
     return aux_ok_t([=](size_t i) -> uint8_t { return L[i]; }, (size_t)p, (size_t)q);
 }
 
-// ---- SWAR helpers for the long fields (SEQ, QUAL) of a line that sits in the staged shared-memory window ----
+// ---- SWAR helpers for the long fields (SEQ, QUAL) ----
 
-// unaligned 32-bit read from shared memory; reads one aligned word past `off` (always inside the dynamic smem block)
-__device__ __forceinline__ uint32_t lds_u32(const uint8_t *text, uint32_t off)
-{
-    const uint8_t *q = text + off;
-    const uint32_t a = (uint32_t)((uintptr_t)q & 3u);                // alignment of the address, not of the offset
-    const uint32_t *p = reinterpret_cast<const uint32_t *>(q - a);
-    return __funnelshift_r(p[0], p[1], a * 8);
-}
 __device__ __forceinline__ uint32_t zero_bytes(uint32_t d)          // 0x80 in every byte of d that is zero (exact)
 {
     return ~(((d & 0x7f7f7f7fu) + 0x7f7f7f7fu) | d | 0x7f7f7f7fu);
@@ -280,166 +278,11 @@ __device__ __forceinline__ uint64_t mix64(uint64_t x)
     return x;
 }
 
-// Parses the line starting at `s` (ending at newline position `e`, e == n for an unterminated last
-// line).  Returns 0 or an SSB_E_* code.  A line is accepted only if htslib's parse -> format round
-// trip (sam_read1 + sam_write1, stochasticSpike.c:248,273) reproduces it byte for byte, so that the
-// emit stage can pass the original bytes through (DESIGN.md "pass-through envelope").
-__device__ int parse_line(const Cursor &cur, size_t s, size_t e, const ContigNames &names, int &tid_cache, SamRec &r)
-{
-    size_t p = s;
-    uint64_t v;
-    r.line_off = s;
-    r.line_len = (uint32_t)(e - s + (e < cur.n ? 1 : 0));
-    r.bits = e < cur.n ? 0 : REC_NO_NL;
-    for (int k = 0; k < 6; k++) r.pad[k] = 0;
-    if (e - s > 0x7fffffffull) return SSB_E_FORMAT;
-    // QNAME
-    uint32_t h1 = 2166136261u, h2 = 0x9747b28cu;
-    while (p < e) { uint32_t c = cur.at(p); if (c == '\t') break; if (c < '!' || c > '~') return SSB_E_FORMAT; h1 = (h1 ^ c) * 16777619u; h2 = (h2 + c) * 0x85ebca6bu; p++; }
-    if (p >= e || p == s || p - s > 254) return SSB_E_FORMAT;
-    r.qhash = ((uint64_t)h1 << 32) | (h2 ^ (h2 >> 15)); r.qname_len = (uint16_t)(p - s);
-    p++;
-    // FLAG
-    if (parse_udec(cur, p, e, 65535, v)) return SSB_E_FORMAT;
-    r.flag = (uint16_t)v; p++;
-    // RNAME
-    size_t p0 = p;
-    while (p < e && cur.at(p) != '\t') p++;
-    if (p >= e || p == p0) return SSB_E_FORMAT;
-    const size_t rname_len = p - p0;
-    if (rname_len == 1 && cur.at(p0) == '*') r.tid = -1;
-    else {
-        r.tid = name_lookup(cur, p0, rname_len, names, tid_cache);
-        if (r.tid < 0) return SSB_E_FORMAT;          // htslib would warn and print '*': not a pass-through
-        tid_cache = r.tid;
-    }
-    p++;
-    // POS
-    if (parse_udec(cur, p, e, 0x7fffffffull, v)) return SSB_E_FORMAT;
-    r.pos = (int32_t)v - 1; p++;
-    // MAPQ
-    if (parse_udec(cur, p, e, 255, v)) return SSB_E_FORMAT;
-    r.mapq = (uint8_t)v; p++;
-    // CIGAR
-    p0 = p;
-    uint64_t rlen = 0, qlen = 0; bool has_cigar = true, simple = true;
-    if (cur.at(p) == '*' && p + 1 < e && cur.at(p + 1) == '\t') { has_cigar = false; simple = false; p++; }
-    else {
-        uint64_t num = 0; int nd = 0; uint8_t first = 0;
-        while (p < e) {
-            uint8_t c = cur.at(p);
-            if (c == '\t') break;
-            if (c >= '0' && c <= '9') { if (!nd) first = c; num = num * 10 + (c - '0'); nd++; if (num > 0x0fffffffull) return SSB_E_FORMAT; }
-            else {
-                if (!nd || (nd > 1 && first == '0')) return SSB_E_FORMAT;
-                switch (c) {
-                case 'M': case '=': case 'X': rlen += num; qlen += num; break;
-                case 'D': case 'N': rlen += num; simple = false; break;
-                case 'I': case 'S': qlen += num; simple = false; break;
-                case 'H': case 'P': simple = false; break;
-                default: return SSB_E_FORMAT;
-                }
-                num = 0; nd = 0;
-            }
-            p++;
-        }
-        if (nd) return SSB_E_FORMAT;
-    }
-    if (simple) r.bits |= REC_SIMPLE;
-    if (p >= e || p == p0 || p - p0 > 65535 || p0 - s > 65535) return SSB_E_FORMAT;
-    r.cigar_off = (uint16_t)(p0 - s); r.cigar_len = has_cigar ? (uint16_t)(p - p0) : 0;
-    if (r.pos < 0 && rlen) return SSB_E_FORMAT;
-    if ((uint64_t)(r.pos < 0 ? 0 : r.pos) + rlen > 0x7ffffff0ull) return SSB_E_FORMAT;
-    r.end = r.pos + (int32_t)rlen;
-    p++;
-    // RNEXT: '*', '=' or another @SQ name (the same name spelled out would be printed back as '=')
-    p0 = p;
-    while (p < e && cur.at(p) != '\t') p++;
-    if (p >= e || p == p0) return SSB_E_FORMAT;
-    if (!(p - p0 == 1 && (cur.at(p0) == '*' || cur.at(p0) == '='))) {
-        int mt = name_lookup(cur, p0, p - p0, names, -1);
-        if (mt < 0 || mt == r.tid) return SSB_E_FORMAT;
-    } else if (cur.at(p0) == '=' && r.tid < 0) return SSB_E_FORMAT;
-    p++;
-    // PNEXT
-    if (parse_udec(cur, p, e, 0x7fffffffull, v)) return SSB_E_FORMAT;
-    p++;
-    // TLEN
-    if (p < e && cur.at(p) == '-') { p++; if (p < e && cur.at(p) == '0') return SSB_E_FORMAT; }
-    if (parse_udec(cur, p, e, 0x7fffffffull, v)) return SSB_E_FORMAT;
-    p++;
-    // SEQ: with a CIGAR its length is the CIGAR's query length, so the field is validated a word at a time
-    r.seq_off = (uint32_t)(p - s);
-    p0 = p;
-    const bool in_smem = e <= cur.lim && s >= cur.base;
-    if (p < e && cur.at(p) == '*' && p + 1 < e && cur.at(p + 1) == '\t') { r.l_seq = 0; p++; }
-    else if (has_cigar && in_smem && qlen > 0 && p + qlen < e) {
-        const uint32_t L = (uint32_t)qlen, off = (uint32_t)(p - cur.base);
-        uint32_t badw = 0;
-        for (uint32_t w = 0; w < L; w += 4) {
-            uint32_t x = lds_u32(cur.smem, off + w);
-            const uint32_t rem = L - w;
-            if (rem < 4) x = (x & ((1u << (8 * rem)) - 1u)) | (0x41414141u << (8 * rem));
-            if (non_acgtn_bytes(x)) { for (int k = 0; k < 4; k++) if (!seq_char_ok((uint8_t)(x >> (8 * k)))) badw = 1; }   // other IUPAC codes, '='
-        }
-        if (badw) return SSB_E_FORMAT;
-        p += L;
-        if (cur.at(p) != '\t') return SSB_E_FORMAT;               // htslib: "CIGAR and query sequence are of different length"
-        r.l_seq = L;
-    } else {
-        while (p < e) { uint8_t c = cur.at(p); if (c == '\t') break; if (!seq_char_ok(c)) return SSB_E_FORMAT; p++; }
-        r.l_seq = (uint32_t)(p - p0);
-        if (has_cigar && qlen != r.l_seq) return SSB_E_FORMAT;
-    }
-    if (p >= e || p == p0) return SSB_E_FORMAT;
-    p++;
-    // QUAL
-    r.qual_off = (uint32_t)(p - s);
-    if (p >= e) return SSB_E_FORMAT;
-    size_t qend;
-    if (cur.at(p) == '*' && (p + 1 == e || cur.at(p + 1) == '\t')) { r.bits |= REC_QUALSTAR; qend = p + 1; }
-    else {
-        qend = p + r.l_seq;
-        if (r.l_seq == 0 || qend > e) return SSB_E_FORMAT;
-        if (qend < e && cur.at(qend) != '\t') return SSB_E_FORMAT;  // htslib: "SEQ and QUAL are of different length"
-        if (in_smem) {
-            const uint32_t L = r.l_seq, off = (uint32_t)(p - cur.base);
-            uint32_t badw = 0;
-            for (uint32_t w = 0; w < L; w += 4) {
-                uint32_t x = lds_u32(cur.smem, off + w);
-                const uint32_t rem = L - w;
-                if (rem < 4) x = (x & ((1u << (8 * rem)) - 1u)) | (0x21212121u << (8 * rem));
-                badw |= nonprint_bytes(x);
-            }
-            if (badw) return SSB_E_FORMAT;
-        } else for (size_t i = p; i < qend; i++) { uint8_t c = cur.at(i); if (c < '!' || c > '~') return SSB_E_FORMAT; }
-    }
-    // optional fields
-    p = qend;
-    while (p < e) {
-        size_t a = p + 1, q = a;                    // cur.at(p) == '\t'
-        while (q < e && cur.at(q) != '\t') q++;
-        { const int ar = aux_ok(cur, a, q); if (ar == AUX_FLOAT) r.bits |= REC_AUX_F; else if (ar) return SSB_E_FORMAT; }
-        p = q;
-    }
-    // read_bam (stochasticSpike.c:253-263) + bam_plp_push's tid test
-    bool pass = !(r.flag & (4 | 256 | 512 | 1024)) && r.mapq >= 30 && !((r.flag & 1) && !(r.flag & 2));
-    if (pass && r.tid >= 0) {
-        r.bits |= REC_PUSHED;
-        if (r.end > r.pos) {
-            if (r.l_seq == 0) return SSB_E_FORMAT;  // a kept read without SEQ makes the reference read outside its buffer
-            r.bits |= REC_KEEP;
-        }
-    }
-    return 0;
-}
+// ---- the careful parser: any line, in the staged tile or in global memory ----
 
-
-
-// ---- the same parser for a line that lies completely inside the staged shared-memory window: 32-bit offsets, direct
-// ---- shared-memory reads, word-at-a-time validation of the long fields.  L = first byte of the line, len = bytes
-// ---- without the newline.  Accepts / rejects exactly what parse_line() does.
-__device__ __forceinline__ int smem_udec(const uint8_t *L, uint32_t &p, uint32_t len, uint32_t maxv, uint32_t &out)
+// Canonical decimal field ending at '\t' (what htslib prints back): digits only, no leading zero unless the value is 0,
+// value <= maxv.  On success p sits on the terminating tab.
+__device__ __forceinline__ int udec(const uint8_t *L, uint32_t &p, uint32_t len, uint32_t maxv, uint32_t &out)
 {
     const uint32_t p0 = p; uint32_t v = 0;
     while (p < len) {
@@ -458,9 +301,10 @@ __device__ __forceinline__ int smem_udec(const uint8_t *L, uint32_t &p, uint32_t
     return 0;
 }
 
-// words of the field [a, a+n) of the line: `bad` accumulates the flagged bytes.  CHECK(x) returns 0x80 flags.
+// words of the field [a, a+n) of the line: `bad` accumulates the flagged bytes.  CHECK(x) returns 0x80 flags.  Only aligned
+// words inside the field are loaded, so the line may lie in shared or in global memory.
 template <typename CHECK>
-__device__ __forceinline__ uint32_t smem_check_field(const uint8_t *L, uint32_t a, uint32_t n, uint32_t filler, CHECK check)
+__device__ __forceinline__ uint32_t check_field(const uint8_t *L, uint32_t a, uint32_t n, uint32_t filler, CHECK check)
 {
     uint32_t bad = 0, i = 0;
     // bytes up to the first 4-byte aligned address, then aligned words, then the tail
@@ -484,7 +328,12 @@ __device__ __forceinline__ uint32_t smem_check_field(const uint8_t *L, uint32_t 
     return bad;
 }
 
-__device__ int parse_line_smem(const Cursor &cur, const uint8_t *L, uint32_t len, size_t s, bool has_nl, const ContigNames &names, int &tid_cache, SamRec &r)
+// Parses the line of len bytes at L (without its newline; has_nl: one follows) that starts at body offset s.  L points into the
+// staged tile or into the body in global memory; every read is at an offset < len, so nothing past the line is touched.
+// Returns 0 or an SSB_E_* code.  A line is accepted only if htslib's parse -> format round trip (sam_read1 + sam_write1,
+// stochasticSpike.c:248,273) reproduces it byte for byte, so that the emit stage can pass the original bytes through
+// (DESIGN.md "pass-through envelope").
+__device__ int parse_line(const uint8_t *L, uint32_t len, size_t s, bool has_nl, const ContigNames &names, int &tid_cache, SamRec &r)
 {
     uint32_t p = 0, v;
     r.line_off = s;
@@ -497,7 +346,7 @@ __device__ int parse_line_smem(const Cursor &cur, const uint8_t *L, uint32_t len
     if (p >= len || p == 0 || p > 254) return SSB_E_FORMAT;
     r.qhash = ((uint64_t)h1 << 32) | (h2 ^ (h2 >> 15)); r.qname_len = (uint16_t)p;
     p++;
-    if (smem_udec(L, p, len, 65535u, v)) return SSB_E_FORMAT;
+    if (udec(L, p, len, 65535u, v)) return SSB_E_FORMAT;
     r.flag = (uint16_t)v; p++;
     // RNAME
     uint32_t p0 = p;
@@ -505,19 +354,19 @@ __device__ int parse_line_smem(const Cursor &cur, const uint8_t *L, uint32_t len
     if (p >= len || p == p0) return SSB_E_FORMAT;
     if (p - p0 == 1 && L[p0] == '*') r.tid = -1;
     else {
-        r.tid = name_lookup(cur, s + p0, p - p0, names, tid_cache);
-        if (r.tid < 0) return SSB_E_FORMAT;
+        r.tid = name_lookup(L + p0, p - p0, names, tid_cache);
+        if (r.tid < 0) return SSB_E_FORMAT;          // htslib would warn and print '*': not a pass-through
         tid_cache = r.tid;
     }
     p++;
-    if (smem_udec(L, p, len, 0x7fffffffu, v)) return SSB_E_FORMAT;
+    if (udec(L, p, len, 0x7fffffffu, v)) return SSB_E_FORMAT;
     r.pos = (int32_t)v - 1; p++;
-    if (smem_udec(L, p, len, 255u, v)) return SSB_E_FORMAT;
+    if (udec(L, p, len, 255u, v)) return SSB_E_FORMAT;
     r.mapq = (uint8_t)v; p++;
     // CIGAR
     p0 = p;
     uint32_t rlen = 0, qlen = 0; bool has_cigar = true, simple = true;
-    if (L[p] == '*' && p + 1 < len && L[p + 1] == '\t') { has_cigar = false; simple = false; p++; }
+    if (p + 1 < len && L[p] == '*' && L[p + 1] == '\t') { has_cigar = false; simple = false; p++; }
     else {
         uint32_t num = 0; int nd = 0; uint32_t first = 0;
         while (p < len) {
@@ -527,13 +376,11 @@ __device__ int parse_line_smem(const Cursor &cur, const uint8_t *L, uint32_t len
             if (d <= 9u) { if (!nd) first = c; num = num * 10u + d; nd++; if (nd > 9 || num > 0x0fffffffu) return SSB_E_FORMAT; }
             else {
                 if (!nd || (nd > 1 && first == '0')) return SSB_E_FORMAT;
-                switch (c) {
-                case 'M': case '=': case 'X': rlen += num; qlen += num; break;
-                case 'D': case 'N': rlen += num; simple = false; break;
-                case 'I': case 'S': qlen += num; simple = false; break;
-                case 'H': case 'P': simple = false; break;
-                default: return SSB_E_FORMAT;
-                }
+                const uint32_t k = cigar_op(c);
+                if (!(k & CIG_OK)) return SSB_E_FORMAT;
+                if (k & CIG_REF) rlen += num;
+                if (k & CIG_QRY) qlen += num;
+                if (!(k & CIG_M)) simple = false;
                 if (rlen > 0x7ffffff0u || qlen > 0x7ffffff0u) return SSB_E_FORMAT;
                 num = 0; nd = 0;
             }
@@ -548,26 +395,26 @@ __device__ int parse_line_smem(const Cursor &cur, const uint8_t *L, uint32_t len
     if ((uint64_t)(r.pos < 0 ? 0 : r.pos) + rlen > 0x7ffffff0ull) return SSB_E_FORMAT;
     r.end = r.pos + (int32_t)rlen;
     p++;
-    // RNEXT
+    // RNEXT: '*', '=' or another @SQ name (the same name spelled out would be printed back as '=')
     p0 = p;
     while (p < len && L[p] != '\t') p++;
     if (p >= len || p == p0) return SSB_E_FORMAT;
     if (!(p - p0 == 1 && (L[p0] == '*' || L[p0] == '='))) {
-        const int mt = name_lookup(cur, s + p0, p - p0, names, -1);
+        const int mt = name_lookup(L + p0, p - p0, names, -1);
         if (mt < 0 || mt == r.tid) return SSB_E_FORMAT;
     } else if (L[p0] == '=' && r.tid < 0) return SSB_E_FORMAT;
     p++;
-    if (smem_udec(L, p, len, 0x7fffffffu, v)) return SSB_E_FORMAT;   // PNEXT
+    if (udec(L, p, len, 0x7fffffffu, v)) return SSB_E_FORMAT;   // PNEXT
     p++;
     if (p < len && L[p] == '-') { p++; if (p < len && L[p] == '0') return SSB_E_FORMAT; }
-    if (smem_udec(L, p, len, 0x7fffffffu, v)) return SSB_E_FORMAT;   // TLEN
+    if (udec(L, p, len, 0x7fffffffu, v)) return SSB_E_FORMAT;   // TLEN
     p++;
     // SEQ
     r.seq_off = p;
     p0 = p;
     if (p < len && L[p] == '*' && p + 1 < len && L[p + 1] == '\t') { r.l_seq = 0; p++; }
     else if (has_cigar && qlen > 0 && p + qlen < len) {
-        const uint32_t bad = smem_check_field(L, p, qlen, 0x41414141u, [](uint32_t x) { return non_acgtn_bytes(x); });
+        const uint32_t bad = check_field(L, p, qlen, 0x41414141u, [](uint32_t x) { return non_acgtn_bytes(x); });
         if (bad) for (uint32_t i = 0; i < qlen; i++) if (!seq_char_ok(L[p + i])) return SSB_E_FORMAT;    // other IUPAC codes, '='
         p += qlen;
         if (L[p] != '\t') return SSB_E_FORMAT;                      // htslib: "CIGAR and query sequence are of different length"
@@ -588,35 +435,30 @@ __device__ int parse_line_smem(const Cursor &cur, const uint8_t *L, uint32_t len
         qend = p + r.l_seq;
         if (r.l_seq == 0 || qend > len) return SSB_E_FORMAT;
         if (qend < len && L[qend] != '\t') return SSB_E_FORMAT;     // htslib: "SEQ and QUAL are of different length"
-        if (smem_check_field(L, p, r.l_seq, 0x21212121u, [](uint32_t x) { return nonprint_bytes(x); })) return SSB_E_FORMAT;
+        if (check_field(L, p, r.l_seq, 0x21212121u, [](uint32_t x) { return nonprint_bytes(x); })) return SSB_E_FORMAT;
     }
     // optional fields
-    for (size_t q = s + qend; q < s + len;) {
-        size_t a = q + 1, b = a;
-        while (b < s + len && cur.at(b) != '\t') b++;
-        { const int ar = aux_ok(cur, a, b); if (ar == AUX_FLOAT) r.bits |= REC_AUX_F; else if (ar) return SSB_E_FORMAT; }
+    for (uint32_t q = qend; q < len;) {
+        uint32_t a = q + 1, b = a;
+        while (b < len && L[b] != '\t') b++;
+        { const int ar = aux_ok(L, a, b); if (ar == AUX_FLOAT) r.bits |= REC_AUX_F; else if (ar) return SSB_E_FORMAT; }
         q = b;
     }
-    // read_bam (stochasticSpike.c:253-263) + bam_plp_push's tid test
-    const bool pass = !(r.flag & (4 | 256 | 512 | 1024)) && r.mapq >= 30 && !((r.flag & 1) && !(r.flag & 2));
-    if (pass && r.tid >= 0) {
-        r.bits |= REC_PUSHED;
-        if (r.end > r.pos) {
-            if (r.l_seq == 0) return SSB_E_FORMAT;
-            r.bits |= REC_KEEP;
-        }
-    }
+    read_bam_filter(r);
+    if ((r.bits & REC_KEEP) && r.l_seq == 0) return SSB_E_FORMAT;  // a kept read without SEQ makes the reference read outside its buffer
     return 0;
 }
 
-// ---- the common shape of a line, parsed so that the lanes of a warp stay together ----
+// ---- the fast parser: the common shape of a line, parsed so that the lanes of a warp stay together ----
 //
-// parse_line_smem() leaves a loop the moment it meets a byte it does not like; with those exits inside the loops the
-// lanes of a warp no longer reconverge after a field whose length differs from lane to lane, and everything behind it --
-// SEQ, QUAL, the comparison with the reference -- runs a few lanes at a time.  The functions below accept exactly the
-// lines of the common shape (mapped RNAME, a CIGAR, RNEXT '=' or '*', SEQ of the CIGAR's query length) and collect
-// every objection in one flag instead of leaving; a line that raises the flag is handed to parse_line_smem(), which
-// decides.  Every loop has one exit, and the lanes meet again (__syncwarp) after each field.
+// The tokeniser has two line parsers: the careful parse_line() above, which decides every line, and this one
+// (parse_head_conv + long_fields) for the first lines of a tile that end inside the staged window.  parse_line() leaves a
+// loop the moment it meets a byte it does not like; with those exits inside the loops the lanes of a warp no longer
+// reconverge after a field whose length differs from lane to lane, and everything behind it -- SEQ, QUAL, the comparison
+// with the reference -- runs a few lanes at a time.  The functions below accept exactly the lines of the common shape
+// (mapped RNAME, a CIGAR, RNEXT '=' or '*', SEQ of the CIGAR's query length) and collect every objection in one flag
+// instead of leaving; a line that raises the flag is handed to parse_line(), which decides.  Every loop has one exit, and
+// the lanes meet again (__syncwarp) after each field.  Both share read_bam_filter() and cigar_op().
 
 __device__ __forceinline__ uint32_t udec_conv(const uint8_t *L, uint32_t &p, uint32_t len, uint32_t maxv, uint32_t &out)
 {
@@ -638,7 +480,7 @@ __device__ __forceinline__ uint32_t udec_conv(const uint8_t *L, uint32_t &p, uin
 
 // QNAME .. QUAL bounds of the line [L, L+len).  Returns 0 when the line has the common shape and its head is valid; then
 // r holds everything but the verdict on the SEQ / QUAL / optional-field bytes, and qend is the end of QUAL.
-__device__ __forceinline__ uint32_t parse_head_conv(const Cursor &cur, const uint8_t *L, uint32_t len, size_t s, bool has_nl,
+__device__ __forceinline__ uint32_t parse_head_conv(const uint8_t *L, uint32_t len, size_t s, bool has_nl,
                                                     const ContigNames &names, int tid_cache, SamRec &r, uint32_t &qend, unsigned mask)
 {
     uint32_t p = 0, v = 0, bad = 0;
@@ -660,7 +502,7 @@ __device__ __forceinline__ uint32_t parse_head_conv(const Cursor &cur, const uin
     bad |= (uint32_t)(p >= len) | (uint32_t)(p == p0);
     __syncwarp(mask);
     r.tid = -1;
-    if (!bad && !(p - p0 == 1 && L[p0] == '*')) r.tid = name_lookup(cur, s + p0, p - p0, names, tid_cache);
+    if (!bad && !(p - p0 == 1 && L[p0] == '*')) r.tid = name_lookup(L + p0, p - p0, names, tid_cache);
     bad |= (uint32_t)(r.tid < 0);
     p++;
     __syncwarp(mask);
@@ -678,11 +520,11 @@ __device__ __forceinline__ uint32_t parse_head_conv(const Cursor &cur, const uin
         if (d <= 9u) { if (!nd) first = c; num = num * 10u + d; nd++; bad |= (uint32_t)(nd > 8u); }           // (eight digits < 2^28; longer: the careful parser decides)
         else {
             bad |= (uint32_t)(!nd) | (uint32_t)(nd > 1u && first == '0');
-            const bool m = c == 'M' || c == '=' || c == 'X', dn = c == 'D' || c == 'N', is = c == 'I' || c == 'S', hp = c == 'H' || c == 'P';
-            if (m || dn) rlen += num;
-            if (m || is) qlen += num;
-            if (!m) simple = false;
-            bad |= (uint32_t)(!(m || dn || is || hp)) | (uint32_t)(rlen > 0x7ffffff0u) | (uint32_t)(qlen > 0x7ffffff0u);
+            const uint32_t k = cigar_op(c);
+            if (k & CIG_REF) rlen += num;
+            if (k & CIG_QRY) qlen += num;
+            if (!(k & CIG_M)) simple = false;
+            bad |= (uint32_t)!(k & CIG_OK) | (uint32_t)(rlen > 0x7ffffff0u) | (uint32_t)(qlen > 0x7ffffff0u);
             num = 0; nd = 0;
         }
         p++;
@@ -717,8 +559,7 @@ __device__ __forceinline__ uint32_t parse_head_conv(const Cursor &cur, const uin
         if (L[p] == '*' && (p + 1 == len || L[p + 1] == '\t')) { r.bits |= REC_QUALSTAR; qend = p + 1; }
         else { qend = p + qlen; bad |= (uint32_t)(qend > len); if (!bad && qend < len) bad |= (uint32_t)(L[qend] != '\t'); }
     }
-    const bool pass = !(r.flag & (4 | 256 | 512 | 1024)) && r.mapq >= 30 && !((r.flag & 1) && !(r.flag & 2));
-    if (pass && r.end > r.pos) r.bits |= REC_PUSHED | REC_KEEP; else if (pass) r.bits |= REC_PUSHED;
+    read_bam_filter(r);
     return bad;
 }
 
@@ -855,7 +696,7 @@ __device__ __forceinline__ void mbar_wait(unsigned long long *bar, uint32_t pari
 }
 
 #ifndef SSB_PARSE_MINBLOCKS
-#define SSB_PARSE_MINBLOCKS 5      // 5 blocks of 128 threads per SM: 96 registers (a few spills in per-tile code) against 112 and 4 blocks
+#define SSB_PARSE_MINBLOCKS 5      // 5 blocks of 128 threads per SM: at most 96 registers, against 112 and 4 blocks
 #endif
 __global__ void __launch_bounds__(THREADS, SSB_PARSE_MINBLOCKS)
 parse_kernel(const uint8_t *__restrict__ body, size_t n, ContigNames names, SamRec *__restrict__ recs, size_t rec_cap,
@@ -1050,11 +891,10 @@ parse_kernel(const uint8_t *__restrict__ body, size_t n, ContigNames names, SamR
         }
         __syncthreads();
         // 4. one line per thread of warps 1..3.  The last line of the tile ends in the overhang (or beyond): warp 0 finds its newline.
-        Cursor cur{text, body, T0, stage_end, n};
         if (wid == 0 && n_here > 0) {
             size_t e = T0 + starts[n_here - 1] + lane;
             for (;;) {
-                const bool hit = e >= n || cur.at(e) == '\n';
+                const bool hit = e >= n || (e < stage_end ? text[e - T0] : body[e]) == '\n';
                 const unsigned m = __ballot_sync(0xffffffffu, hit);
                 if (m) { e = e - lane + (__ffs(m) - 1); break; }
                 e += 32;
@@ -1068,7 +908,7 @@ parse_kernel(const uint8_t *__restrict__ body, size_t n, ContigNames names, SamR
             if (lane == 0) { s_base = excl; if (tile == n_tiles - 1) *n_lines_out = excl + n_here; }
         }
         // 4a. heads.  The threads of warps 1..3 take one line each; the lanes of a warp stay together (parse_head_conv).  A line that
-        //     is not of the common shape, or does not end inside the staged window, is parsed by the careful functions at once.
+        //     is not of the common shape, or does not end inside the staged window, is parsed by the careful parser at once.
         constexpr uint32_t PARSERS = THREADS - 32;                         // warp 0 serves (look-back, last newline); the others parse.  (Giving warp 0 a
         // quarter of the lines after its service was measured: 12.6 ms instead of 11.7 -- its lines start late whenever the look-back has to wait.)
         const uint32_t li = wid ? (uint32_t)(lane * (THREADS / 32 - 1) + (wid - 1)) : 0xffffffffu;   // consecutive lines go to different warps
@@ -1078,13 +918,11 @@ parse_kernel(const uint8_t *__restrict__ body, size_t n, ContigNames names, SamR
         if (have) {
             lo = starts[li]; ls = T0 + lo;
             const size_t e = (li + 1 < n_here) ? T0 + starts[li + 1] - 1 : (size_t)s_last_end;
-            const bool insm = e <= stage_end && e - ls < 0x40000000ull;
+            const bool insm = e <= stage_end;
             const unsigned fmask = __ballot_sync(wmask, insm);
-            if (insm) {
-                len = (uint32_t)(e - ls);
-                fast = parse_head_conv(cur, text + lo, len, ls, e < n, names, tid_cache, r, qend, fmask) == 0;
-                if (!fast) rc = parse_line_smem(cur, text + lo, len, ls, e < n, names, tid_cache, r);
-            } else rc = parse_line(cur, ls, e, names, tid_cache, r);
+            len = (uint32_t)(e - ls);
+            if (insm) fast = parse_head_conv(text + lo, len, ls, e < n, names, tid_cache, r, qend, fmask) == 0;
+            if (!fast) rc = e - ls > 0x7fffffffull ? SSB_E_FORMAT : parse_line(insm ? text + lo : body + ls, len, ls, e < n, names, tid_cache, r);
             if (!rc && r.tid >= 0) tid_cache = r.tid;
         }
         // the reference window under the tile's reads: lowest (tid, pos) among the reads that align 1:1
@@ -1103,16 +941,12 @@ parse_kernel(const uint8_t *__restrict__ body, size_t n, ContigNames names, SamR
         for (uint32_t i = wid ? li + PARSERS : 0xffffffffu; i < n_here; i += PARSERS) {
             const size_t s = T0 + starts[i];
             const size_t e = (i + 1 < n_here) ? T0 + starts[i + 1] - 1 : (size_t)s_last_end;
-            SamRec r2; int rc2;
-            if (e <= stage_end && e - s < 0x40000000ull) rc2 = parse_line_smem(cur, text + (s - T0), (uint32_t)(e - s), s, e < n, names, tid_cache, r2);
-            else rc2 = parse_line(cur, s, e, names, tid_cache, r2);
-            if (rc2) { if (atomicCAS(&err->code, 0, rc2) == 0) err->where = s; memset(&r2, 0, sizeof r2); r2.line_off = s; r2.tid = -1; }
-            shard_keep(r2, names);
+            SamRec r2;
+            const int rc2 = e - s > 0x7fffffffull ? SSB_E_FORMAT
+                                                  : parse_line(e <= stage_end ? text + (s - T0) : body + s, (uint32_t)(e - s), s, e < n, names, tid_cache, r2);
+            store_line(r2, rc2, s, gbase + i, names, recs, rec_cap, err);
             if (r2.bits & REC_KEEP) { atomicAdd(names.n_keep, 1ull); if (r2.end > end_max) end_max = r2.end; }
             if (r2.bits & REC_AUX_F) atomicAdd(names.n_float, 1ull);
-            const unsigned long long g2 = gbase + i;
-            if (g2 < rec_cap) { recs[g2] = r2; line_keys(names, g2, r2); }
-            else if (atomicCAS(&err->code, 0, SSB_E_NOMEM) == 0) err->where = s;
         }
         bool in_win = false; int32_t w_lo = 0; int wtid = -1;
         if (names.exc) {
@@ -1152,16 +986,13 @@ parse_kernel(const uint8_t *__restrict__ body, size_t n, ContigNames names, SamR
                 for (uint32_t q = qend; q < len;) {                      // optional fields, straight from shared memory
                     uint32_t a = q + 1, b = a;
                     while (b < len && L[b] != '\t') b++;
-                    { const int ar = aux_ok_smem(L, a, b); if (ar == AUX_FLOAT) r.bits |= REC_AUX_F; else if (ar) bad = 1; }
+                    { const int ar = aux_ok(L, a, b); if (ar == AUX_FLOAT) r.bits |= REC_AUX_F; else if (ar) bad = 1; }
                     q = b;
                 }
                 if (bad) rc = SSB_E_FORMAT;
             }
-            if (rc) { if (atomicCAS(&err->code, 0, rc) == 0) err->where = ls; memset(&r, 0, sizeof r); r.line_off = ls; r.tid = -1; }
-            shard_keep(r, names);
+            store_line(r, rc, ls, gi, names, recs, rec_cap, err);
             if ((r.bits & REC_KEEP) && r.end > end_max) end_max = r.end;
-            if (gi < rec_cap) { recs[gi] = r; line_keys(names, gi, r); }
-            else if (atomicCAS(&err->code, 0, SSB_E_NOMEM) == 0) err->where = ls;
         }
         {   // kept lines of this tile: one atomic per warp
             const unsigned km = __ballot_sync(0xffffffffu, have && (r.bits & REC_KEEP));

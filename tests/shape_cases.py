@@ -532,9 +532,10 @@ def chain_case(outdir, seed, size, seq_star=False):
 
 
 def tokeniser_paths(body: bytes):
-    """Which line parser of parse_kernel (sam_parse.cuh) meets each line of `body`: 'conv' (the common-shape parser; a line it
-    objects to goes on to the staged careful parser), 'staged' (the careful parser over the staged tile: lines beyond the first
-    PARSERS of a tile) or 'global' (the careful parser over global memory: lines that end past the tile's overhang).
+    """Which route through parse_kernel's two line parsers (sam_parse.cuh) each line of `body` takes: 'conv' (the common-shape
+    parser; a line it objects to goes on to the careful parser over the staged tile), 'staged' (the careful parser over the
+    staged tile: lines beyond the first PARSERS of a tile) or 'global' (the careful parser over global memory: lines that end
+    past the tile's overhang).
     Returns [(line start, path)]."""
     n = len(body)
     starts = [0] + [i + 1 for i in range(n) if body[i] == 10 and i + 1 < n]

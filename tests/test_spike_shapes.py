@@ -11,7 +11,8 @@ restatement and the shim state them (SURVEY App. D): they have not been checked 
 
 CPU: the builder places every shape and every kind of target, writes lines inside the pass-through envelope in coordinate
 order, the restatement accepts every input and keeps exactly the lines read_bam's filter keeps, and the shifted inputs put
-kept lines on each of the tokeniser's three line parsers."""
+kept lines on each of the tokeniser's three routes: its fast parser, and its careful parser over the staged tile and over
+global memory."""
 import os
 import re
 
@@ -120,8 +121,8 @@ def test_restatement_accepts_and_keeps_what_the_filter_keeps(name, seed, shift, 
 
 def test_shifts_put_kept_lines_on_every_tokeniser_path(tmp_path):
     """The shifted mixed inputs move every line against the 32 KiB tiles: kept MAPQ-30 lines, kept QUAL '*' lines and kept lines
-    with H / P reach the common-shape parser, the staged careful parser (lines beyond the tile's parsing threads) and the global
-    careful parser (lines that end past the staged overhang), so a slip in any one copy of the filter or of the CIGAR switch shows."""
+    with H / P reach the common-shape parser, the careful parser over the staged tile (lines beyond the tile's parsing threads) and
+    the careful parser over global memory (lines that end past the staged overhang), so a slip on any route shows."""
     seen = {"mapq30": set(), "qualstar": set(), "hp": set()}
     global_shifts = 0
     for k in SHIFTS:
