@@ -356,33 +356,20 @@ __device__ __forceinline__ void emit_edges(const EmitJob &j, int lane)
     if (lane == 0 && j.add_nl) j.dst[j.len] = '\n';
 }
 
-template <int NL, int MINB>
-__global__ void __launch_bounds__(256, MINB)
+// one output line per warp
+__global__ void __launch_bounds__(256, 8)
 emit_kernel(const uint8_t *__restrict__ sam, size_t n_sam, const EmitDesc *__restrict__ desc, const unsigned long long *__restrict__ out_off, size_t K,
             uint8_t *__restrict__ out)
 {
     const int lane = threadIdx.x & 31;
     const size_t warps = ((size_t)gridDim.x * blockDim.x) >> 5;
     const uint8_t *sam_end = sam + n_sam;
-    for (size_t o = (((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5); o < K; o += NL * warps) {
-        EmitJob j[NL]; bool have[NL], in[NL]; uint4 A[NL], B[NL];
-#pragma unroll
-        for (int l = 0; l < NL; l++) {
-            const size_t ol = o + (size_t)l * warps;
-            have[l] = ol < K;
-            j[l] = emit_job(sam, desc[have[l] ? ol : o], out_off[have[l] ? ol : o], out);
-            in[l] = have[l] && (uint32_t)lane < j[l].nvec;
-        }
-#pragma unroll
-        for (int l = 0; l < NL; l++) if (in[l]) emit_load(j[l], lane, sam_end, A[l], B[l]);
-#pragma unroll
-        for (int l = 0; l < NL; l++) if (in[l]) emit_store(j[l], lane, A[l], B[l]);
-#pragma unroll
-        for (int l = 0; l < NL; l++) {
-            if (!have[l]) continue;
-            for (uint32_t i = lane + 32; i < j[l].nvec; i += 32) { emit_load(j[l], i, sam_end, A[l], B[l]); emit_store(j[l], i, A[l], B[l]); }
-            emit_edges(j[l], lane);
-        }
+    for (size_t o = (((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5); o < K; o += warps) {
+        const EmitJob j = emit_job(sam, desc[o], out_off[o], out);
+        uint4 A, B;
+        if ((uint32_t)lane < j.nvec) { emit_load(j, lane, sam_end, A, B); emit_store(j, lane, A, B); }
+        for (uint32_t i = lane + 32; i < j.nvec; i += 32) { emit_load(j, i, sam_end, A, B); emit_store(j, i, A, B); }
+        emit_edges(j, lane);
     }
 }
 

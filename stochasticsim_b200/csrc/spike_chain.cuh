@@ -378,7 +378,6 @@ constexpr size_t P1_SMEM = (size_t)(P1_EW_CAP + P1_CW_CAP) * sizeof(uint4);
 // the cursor), `nonend`: those of them that ended no locus.  A locus that finds no ending draw in the window (y = 0) takes the rest of
 // the window and stays the current locus of the next step; later stages then see a full `done` and change nothing.
 constexpr int P1_STAGES = 6;
-template <int P1_STAGES_T>
 __device__ __forceinline__ int walk_seg(const SegPlanes &P, uint32_t &gr, const uint32_t gto, uint32_t &kr)
 {
     while (gr + 32u <= gto) {                                             // a full window of loci ahead
@@ -389,7 +388,7 @@ __device__ __forceinline__ int walk_seg(const SegPlanes &P, uint32_t &gr, const 
         const uint32_t c0 = __funnelshift_r(ca.x, cb.x, b), c1 = __funnelshift_r(ca.y, cb.y, b), cx = __funnelshift_r(ca.z, cb.z, b);
         uint32_t done = 0u, nonend = 0u, skew = 0u;
 #pragma unroll
-        for (int s = 0; s < P1_STAGES_T; s++) {
+        for (int s = 0; s < P1_STAGES; s++) {
             const uint32_t s0 = c0 << skew, s1 = c1 << skew, sx = cx << skew;      // locus gr + i - skew stands at draw kr + i
             const uint32_t term = (((e0 ^ s0) | (e1 ^ s1) | sx) & ~ej) | done;     // bit i: draw kr+i ends its locus (or is behind the cursor)
             const uint32_t z = ~term & (term + 1u);                                // first draw that does not (0: none, the window is used up)
@@ -399,7 +398,7 @@ __device__ __forceinline__ int walk_seg(const SegPlanes &P, uint32_t &gr, const 
             const uint32_t y = above & (0u - above);                               // the first of them (0: none in this window)
             nonend |= y - z;                                                       // draws [z, y) ended nothing (y = 0: from z to the top)
             done = y | (y - 1u);                                                   // cursor behind y (y = 0: behind the window)
-            if (s + 1 < P1_STAGES_T) skew = (uint32_t)__popc(nonend);
+            if (s + 1 < P1_STAGES) skew = (uint32_t)__popc(nonend);
         }
         const uint32_t d = (uint32_t)__popc(done);
         kr += d; gr += d - (uint32_t)__popc(nonend);
@@ -426,7 +425,6 @@ __device__ __forceinline__ int walk_seg(const SegPlanes &P, uint32_t &gr, const 
 }
 
 // walk [g, g_to) including the targets inside, counting draws only
-template <int ST>
 __device__ int dry_walk(const ChainArgs &A, const SegPlanes &P, int64_t g, const int64_t g_to, size_t h, unsigned long long &k)
 {
     if (k < P.kb) return CHAIN_COMPLEX;
@@ -434,13 +432,13 @@ __device__ int dry_walk(const ChainArgs &A, const SegPlanes &P, int64_t g, const
     int rc = 0;
     while (h < A.H && A.hits[h].locus_index < g_to) {
         const int64_t gt = A.hits[h].locus_index;
-        if ((rc = walk_seg<ST>(P, gr, (uint32_t)(gt - P.gb), kr))) return rc;
+        if ((rc = walk_seg(P, gr, (uint32_t)(gt - P.gb), kr))) return rc;
         k = P.kb + kr;
         if ((rc = dry_apply(A, h, gt, k))) return rc;
         if (k - P.kb >= ((unsigned long long)P.we_n << 5)) return (k + 96ull > P.M) ? CHAIN_OVERRUN : CHAIN_COMPLEX;
         kr = (uint32_t)(k - P.kb); gr = (uint32_t)(gt + 1 - P.gb); h++;
     }
-    if ((rc = walk_seg<ST>(P, gr, (uint32_t)(g_to - P.gb), kr))) return rc;
+    if ((rc = walk_seg(P, gr, (uint32_t)(g_to - P.gb), kr))) return rc;
     k = P.kb + kr;
     return 0;
 }
@@ -454,7 +452,6 @@ struct BoundaryList { unsigned long long off; uint32_t cnt; uint32_t pad; };
 __device__ __forceinline__ uint32_t isqrt_up(uint32_t x) { uint32_t r = (uint32_t)sqrtf((float)x) + 1u; return r; }
 
 // One block per slice.  kbuf/lobuf: two ping-pong halves of `stride` slots each.
-template <int ST>
 __global__ void __launch_bounds__(P1_THREADS)      // (forcing 12 blocks per SM = 40 registers was measured: 12.6 ms instead of 11.7)
 phase1_kernel(ChainArgs A, int64_t L, const GroupDesc *__restrict__ groups, const SliceDesc *__restrict__ slices,
               unsigned long long *__restrict__ kbuf, uint32_t *__restrict__ lobuf, unsigned long long stride,
@@ -520,7 +517,7 @@ phase1_kernel(ChainArgs A, int64_t L, const GroupDesc *__restrict__ groups, cons
         unsigned long long tmin = ~0ull, tmax = 0ull;
         for (uint32_t i = tid; i < alive; i += P1_THREADS) {
             unsigned long long k = kb[cur][i];
-            bad |= dry_walk<ST>(A, SP, g, gc, h0, k);
+            bad |= dry_walk(A, SP, g, gc, h0, k);
             kb[cur][i] = k;
             if (k < tmin) tmin = k;
             if (k > tmax) tmax = k;

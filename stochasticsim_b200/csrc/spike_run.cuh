@@ -1,31 +1,34 @@
-// spike_run.cuh -- one run of the spike path over one shard of the input: the order of the stages, the two streams they
-// run on, and the few points where the host has to look at a number.  (Included at the end of spike.cu.)
+// spike_run.cuh -- one run of the spike path over one shard of the input: the order of its stages on the context's stream,
+// and the few points where the host has to look at a number.  (Included at the end of spike.cu.)
 //
-// Stages (M = main stream, A = second stream; "sync" = the host waits for a handful of scalars that a kernel wrote into
-// mapped pinned memory -- no copy engine is involved, so these waits do not queue behind bulk transfers):
+// Stages, in issue order ("sync" = the host waits for a handful of scalars that a kernel wrote into mapped pinned memory --
+// no copy engine is involved, so these waits do not queue behind the bulk transfers of a streamed run):
 //
-//   M  parse ........................................................ sync 1: lines, kept reads, first error
-//   M  keep flags, sortedness, compaction
-//   A    output order (radix sort by end), output offsets, EMIT        | the output branch: DRAM bound, runs beside
-//   M  mates, coverage runs ......................................... sync 2: runs, covered loci, fold, max span
-//   M  per-locus start/end counts, max depth, local target bounds
-//   A    tallies of the non-target loci (exception list + generic)     | ... the chain branch, which is issue bound
+//   parse ........................................................ sync 1: lines, kept reads, first error
+//   keep flags, sortedness, compaction
+//   output order (radix sort by end), output offsets
+//   mates, coverage runs ......................................... sync 2: runs, covered loci, fold, max span
+//   per-locus start/end counts, max depth, local target bounds
 //      [shards: all-gather summaries, max-reduce the target bounds]
-//   M  target scan, hits, pileup sizes ............................... sync 3: hits, pileup entries
-//   M  pileup gather, reference classes, expected draws .............. sync 4: means / variances -> window geometry (host)
+//   target scan, hits, pileup sizes ............................... sync 3: hits, pileup entries
+//   pileup gather, reference classes, expected draws .............. sync 4: means / variances -> window geometry (host)
+//   EMIT, tallies of the non-target loci (exception list + generic)
 //      [shards: all-gather expected draws -> window centre of this shard]
-//   M  rand() stream, phase 1 (window maps), [shards: precompose]
+//   rand() stream, phase 1 (window maps), [shards: precompose]
 //      [shards: receive the exact offset, look the exit offset up (sync), send it on]
-//   M  compose, chunk boundaries, phase 3 (apply) .................... sync 5: flags (fallbacks: serial chain)
+//   compose, chunk boundaries, phase 3 (apply) .................... sync 5: flags (fallbacks: serial chain)
 //      [shards: agree that nobody changed an offset after sending it; forward spiked bases of straddling reads]
-//   M  join A; patches; SEQ_ERROR records ............................ sync 6: record count; results back
+//   patches; SEQ_ERROR records .................................... sync 6: record count; results back
+//
+// Everything runs on one stream: emit and the tallies beside the chain kernels slowed both down by more than the overlap
+// gave (DESIGN.md section 7).
 #include "exchange.cuh"
 #include <chrono>
 #include <string>
 
 namespace {
 
-struct RunScalars {                 // written by kernels of the main stream, mirrored to the host on demand
+struct RunScalars {                 // written by kernels of the run, mirrored to the host on demand
     unsigned long long n_lines, n_keep, exc_count, n_float;
     DevErr err;
     unsigned long long fold; unsigned int maxspan, maxdepth;
@@ -36,8 +39,6 @@ struct RunScalars {                 // written by kernels of the main stream, mi
     unsigned long long n_se, first_strad, halo_lines, miss[2];
     long long carry_t, carry_h;
     unsigned long long max_end;
-};
-struct RunScalarsA {                // written by kernels of the second stream
     unsigned long long total_out, n_owned;
 };
 
@@ -222,9 +223,8 @@ struct ssb_spike {
     RngTables *d_rng_tab;
     ssb_seq_error *d_se; size_t n_se;          // SEQ_ERROR records of the last run (device resident until asked for)
     // run plumbing
-    cudaStream_t sA;                           // second stream: the output branch and the tallies
-    cudaEvent_t ev_pub, ev_pubA, ev_k, ev_sort, ev_outoff, ev_emit, ev_cover, ev_tally, ev_t[16];
-    RunScalars *d_sc, *h_sc; RunScalarsA *d_scA, *h_scA;       // device scalars and their mapped pinned mirrors
+    cudaEvent_t ev_pub, ev_t[16];
+    RunScalars *d_sc, *h_sc;                   // device scalars and their mapped pinned mirror
     uint8_t *h_map; size_t h_map_bytes;        // mapped pinned scratch: descriptors kernels read, small arrays kernels write
     DevTarget *d_tg; std::vector<DevTarget> tg_host;           // targets of the last run (uploaded again only when they change)
     std::vector<std::string> names;                            // @SQ names (host copy: the streamed run cuts the body by coordinate)
@@ -246,10 +246,8 @@ void spike_free(ssb_spike *sp)
     if (sp->d_lens) cudaFree(sp->d_lens);
     if (sp->d_rng_tab) cudaFree(sp->d_rng_tab);
     if (sp->d_sc) cudaFree(sp->d_sc);
-    if (sp->d_scA) cudaFree(sp->d_scA);
     if (sp->d_tg) cudaFree(sp->d_tg);
     if (sp->h_sc) cudaFreeHost(sp->h_sc);
-    if (sp->h_scA) cudaFreeHost(sp->h_scA);
     if (sp->h_map) cudaFreeHost(sp->h_map);
     if (sp->h_res) cudaFreeHost(sp->h_res);
     for (int i = 0; i < 3; i++) if (sp->st_staging[i]) cudaFree(sp->st_staging[i]);
@@ -257,9 +255,7 @@ void spike_free(ssb_spike *sp)
     for (cudaEvent_t e : sp->st_ev) if (e) cudaEventDestroy(e);
     if (sp->st_out) cudaStreamDestroy(sp->st_out);
     for (auto &c : sp->se_chunks) if (c.first) cudaFree(c.first);
-    if (sp->sA) cudaStreamDestroy(sp->sA);
-    cudaEvent_t *evs[] = {&sp->ev_pub, &sp->ev_pubA, &sp->ev_k, &sp->ev_sort, &sp->ev_outoff, &sp->ev_emit, &sp->ev_cover, &sp->ev_tally};
-    for (cudaEvent_t *e : evs) if (*e) cudaEventDestroy(*e);
+    if (sp->ev_pub) cudaEventDestroy(sp->ev_pub);
     for (int i = 0; i < 16; i++) if (sp->ev_t[i]) cudaEventDestroy(sp->ev_t[i]);
     delete sp;
 }
@@ -277,8 +273,8 @@ extern "C" int ssb_spike_create(ssb_ctx *ctx, const ssb_contig *contigs, int n_c
     sp->st_slot = 0; sp->st_out = NULL;
     for (int i = 0; i < n_contigs; i++) sp->names.push_back(contigs[i].name ? contigs[i].name : "");
     sp->d_names = NULL; sp->d_name_off = NULL; sp->d_seq_ptrs = NULL; sp->d_lens = NULL; sp->d_rng_tab = NULL;
-    sp->sA = NULL; sp->d_sc = sp->h_sc = NULL; sp->d_scA = sp->h_scA = NULL; sp->h_map = NULL; sp->h_map_bytes = 0; sp->d_tg = NULL;
-    sp->ev_pub = sp->ev_pubA = sp->ev_k = sp->ev_sort = sp->ev_outoff = sp->ev_emit = sp->ev_cover = sp->ev_tally = NULL;
+    sp->d_sc = sp->h_sc = NULL; sp->h_map = NULL; sp->h_map_bytes = 0; sp->d_tg = NULL;
+    sp->ev_pub = NULL;
     for (int i = 0; i < 16; i++) sp->ev_t[i] = NULL;
     // every exit below releases what has been allocated so far
 #define SPK_CREATE(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { snprintf(ctx->err, sizeof ctx->err, "%s:%d: %s: %s", __FILE__, __LINE__, #call, cudaGetErrorString(e_)); spike_free(sp); return SSB_E_CUDA; } } while (0)
@@ -296,7 +292,7 @@ extern "C" int ssb_spike_create(ssb_ctx *ctx, const ssb_contig *contigs, int n_c
         } else sp->d_seqs.push_back(d);
         ptrs.push_back(d); lens.push_back(d ? contigs[i].len : 0);
     }
-    { int occ = 1; SPK_CREATE(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, phase1_kernel<P1_STAGES>, P1_THREADS, P1_SMEM)); sp->p1_resident = occ * ctx->sm_count; }
+    { int occ = 1; SPK_CREATE(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, phase1_kernel, P1_THREADS, P1_SMEM)); sp->p1_resident = occ * ctx->sm_count; }
     SPK_CREATE(cudaMalloc(&sp->d_names, names.size() + 1));
     SPK_CREATE(cudaMalloc(&sp->d_name_off, off.size() * sizeof(uint32_t)));
     SPK_CREATE(cudaMalloc(&sp->d_seq_ptrs, (ptrs.size() + 1) * sizeof(uint8_t *)));
@@ -320,19 +316,11 @@ extern "C" int ssb_spike_create(ssb_ctx *ctx, const ssb_contig *contigs, int n_c
     if (e1 == cudaSuccess) e1 = cudaMemcpy(sp->d_rng_tab, tab, sizeof(RngTables), cudaMemcpyHostToDevice);
     delete tab;
     SPK_CREATE(e1);
-    // streams, events, mapped scalars
-    {   // the output branch yields to the chain branch wherever both have blocks waiting
-        int lo_prio = 0, hi_prio = 0;
-        SPK_CREATE(cudaDeviceGetStreamPriorityRange(&lo_prio, &hi_prio));
-        SPK_CREATE(cudaStreamCreateWithPriority(&sp->sA, cudaStreamNonBlocking, lo_prio));
-    }
-    cudaEvent_t *evs[] = {&sp->ev_pub, &sp->ev_pubA, &sp->ev_k, &sp->ev_sort, &sp->ev_outoff, &sp->ev_emit, &sp->ev_cover, &sp->ev_tally};
-    for (cudaEvent_t *e : evs) SPK_CREATE(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
+    // events, mapped scalars
+    SPK_CREATE(cudaEventCreateWithFlags(&sp->ev_pub, cudaEventDisableTiming));
     for (int i = 0; i < 16; i++) SPK_CREATE(cudaEventCreate(&sp->ev_t[i]));
     SPK_CREATE(cudaMalloc(&sp->d_sc, sizeof(RunScalars)));
-    SPK_CREATE(cudaMalloc(&sp->d_scA, sizeof(RunScalarsA)));
     SPK_CREATE(cudaHostAlloc((void **)&sp->h_sc, sizeof(RunScalars), cudaHostAllocMapped));
-    SPK_CREATE(cudaHostAlloc((void **)&sp->h_scA, sizeof(RunScalarsA), cudaHostAllocMapped));
     sp->h_map_bytes = (size_t)32 << 20;
     SPK_CREATE(cudaHostAlloc((void **)&sp->h_map, sp->h_map_bytes, cudaHostAllocMapped));
 #undef SPK_CREATE
@@ -345,7 +333,6 @@ extern "C" void ssb_spike_destroy(ssb_spike *sp)
     if (!sp) return;
     cudaSetDevice(sp->ctx->device);
     cudaStreamSynchronize(sp->ctx->stream);
-    if (sp->sA) cudaStreamSynchronize(sp->sA);
     spike_free(sp);
 }
 
@@ -405,10 +392,7 @@ int run_shard(ssb_spike *sp, const ShardPlan &pl, const uint8_t *d_sam, size_t n
 {
     ssb_ctx *ctx = sp->ctx;
     SSB_CUDA(ctx, cudaSetDevice(ctx->device));
-    // SSB_SCHED: 0 = one stream, every stage in issue order; 1 = output branch (emit, tallies) on the second stream beside phase 1;
-    // 2 = only the tallies beside phase 1, the copy of the text on the main stream in front of it
-    const int sched = getenv("SSB_SCHED") ? atoi(getenv("SSB_SCHED")) : 0;
-    cudaStream_t s = ctx->stream, sA = sched == 0 ? ctx->stream : sp->sA;
+    cudaStream_t s = ctx->stream;
     memset(stats, 0, sizeof *stats);
     *out_bytes = 0;
     const char *dbg_env = getenv("SSB_CHAIN_DEBUG");
@@ -425,26 +409,18 @@ int run_shard(ssb_spike *sp, const ShardPlan &pl, const uint8_t *d_sam, size_t n
     sp->n_se = 0;
     if (!pl.seq) { for (auto &c : sp->se_chunks) if (c.first) cudaFreeAsync(c.first, s); sp->se_chunks.clear(); sp->se_chunked = false; }
     stats->in_bytes = (int64_t)n;
-    Arena ar(s), arA(sA);
-    // declared after the arenas, so destroyed first: nothing may still run when the arenas give their memory back
-    struct Drain { cudaStream_t a, b; ~Drain() { cudaStreamSynchronize(a); cudaStreamSynchronize(b); } } drain{s, sA};
+    Arena ar(s);
+    // declared after the arena, so destroyed first: nothing may still run when the arena gives its memory back
+    struct Drain { cudaStream_t s; ~Drain() { cudaStreamSynchronize(s); } } drain{s};
 
     RunScalars *dsc = sp->d_sc; volatile RunScalars *hsc = sp->h_sc;
-    RunScalarsA *dscA = sp->d_scA; volatile RunScalarsA *hscA = sp->h_scA;
-    RunScalars *hsc_dev = NULL; RunScalarsA *hscA_dev = NULL; uint8_t *hmap_dev = NULL;
+    RunScalars *hsc_dev = NULL; uint8_t *hmap_dev = NULL;
     SSB_CUDA(ctx, cudaHostGetDevicePointer((void **)&hsc_dev, sp->h_sc, 0));
-    SSB_CUDA(ctx, cudaHostGetDevicePointer((void **)&hscA_dev, sp->h_scA, 0));
     SSB_CUDA(ctx, cudaHostGetDevicePointer((void **)&hmap_dev, sp->h_map, 0));
-    auto publish = [&]() -> int {               // main-stream scalars -> host, and wait for them
+    auto publish = [&]() -> int {               // scalars -> host, and wait for them
         SSB_LAUNCH(ctx, copy_words_kernel, 1, 64, 0, s, (const uint32_t *)dsc, (uint32_t *)hsc_dev, (unsigned int)(sizeof(RunScalars) / 4));
         SSB_CUDA(ctx, cudaEventRecord(sp->ev_pub, s));
         SSB_CUDA(ctx, cudaEventSynchronize(sp->ev_pub));
-        return SSB_OK;
-    };
-    auto publishA = [&]() -> int {
-        SSB_LAUNCH(ctx, copy_words_kernel, 1, 64, 0, sA, (const uint32_t *)dscA, (uint32_t *)hscA_dev, (unsigned int)(sizeof(RunScalarsA) / 4));
-        SSB_CUDA(ctx, cudaEventRecord(sp->ev_pubA, sA));
-        SSB_CUDA(ctx, cudaEventSynchronize(sp->ev_pubA));
         return SSB_OK;
     };
     auto fail_dev = [&](const char *stage) -> int {
@@ -459,7 +435,7 @@ int run_shard(ssb_spike *sp, const ShardPlan &pl, const uint8_t *d_sam, size_t n
         if (map_used + bytes > sp->h_map_bytes) {
             // grow: nothing handed out earlier in this run may still be in use -> only allowed before the first hand-out
             if (map_used) { snprintf(ctx->err, sizeof ctx->err, "spike: mapped scratch exhausted"); return SSB_E_NOMEM; }
-            SSB_CUDA(ctx, cudaStreamSynchronize(s)); SSB_CUDA(ctx, cudaStreamSynchronize(sA));
+            SSB_CUDA(ctx, cudaStreamSynchronize(s));
             cudaFreeHost(sp->h_map); sp->h_map = NULL; sp->h_map_bytes = 0;
             SSB_CUDA(ctx, cudaHostAlloc((void **)&sp->h_map, bytes + ((size_t)4 << 20), cudaHostAllocMapped));
             sp->h_map_bytes = bytes + ((size_t)4 << 20);
@@ -470,7 +446,6 @@ int run_shard(ssb_spike *sp, const ShardPlan &pl, const uint8_t *d_sam, size_t n
     };
 
     SSB_CUDA(ctx, cudaMemsetAsync(dsc, 0, sizeof(RunScalars), s));
-    SSB_CUDA(ctx, cudaMemsetAsync(dscA, 0, sizeof(RunScalarsA), sA));
     SSB_CUDA(ctx, cudaMemsetAsync(&dsc->first_strad, 0xff, sizeof(unsigned long long), s));
     const unsigned int odd_cap = 1u << 16;
     OddPatch *d_odd = ar.get<OddPatch>(odd_cap); SPK_CHECK_ARENA(ar);
@@ -537,67 +512,43 @@ int run_shard(ssb_spike *sp, const ShardPlan &pl, const uint8_t *d_sam, size_t n
         if (pl.halo_bytes) SSB_LAUNCH(ctx, halo_lines_kernel, 1, 32, 0, s, recs, N, (unsigned long long)pl.halo_bytes, d_halo_lines);
         if (K && (pl.count > 1 || seq)) SSB_LAUNCH(ctx, first_strad_kernel, grid_for(K, 256), 256, 0, s, k_end, k_rec, recs, K, rg, &dsc->first_strad);
     }
-    SSB_CUDA(ctx, cudaEventRecord(sp->ev_k, s));
     SSB_CUDA(ctx, cudaEventRecord(sp->ev_t[2], s));
 
-    // ---------------------------------------------------------------- A: output order + emit (beside the chain branch)
+    // ---------------------------------------------------------------- output order, output offsets
     uint32_t *perm = NULL; unsigned long long *s_end = NULL, *out_off = NULL, *ord_off = NULL;
     EmitDesc *d_edesc = NULL;
-    SSB_CUDA(ctx, cudaStreamWaitEvent(sA, sp->ev_k, 0));
     if (K) {
         int rc;
-        uint32_t *iota = arA.get<uint32_t>(K); perm = arA.get<uint32_t>(K); s_end = arA.get<unsigned long long>(K);
-        unsigned long long *olen = arA.get<unsigned long long>(K); out_off = arA.get<unsigned long long>(K + 1); ord_off = arA.get<unsigned long long>(K);
-        EmitDesc *edesc = arA.get<EmitDesc>(K);
-        SPK_CHECK_ARENA(arA);
+        uint32_t *iota = ar.get<uint32_t>(K); perm = ar.get<uint32_t>(K); s_end = ar.get<unsigned long long>(K);
+        unsigned long long *olen = ar.get<unsigned long long>(K); out_off = ar.get<unsigned long long>(K + 1); ord_off = ar.get<unsigned long long>(K);
+        d_edesc = ar.get<EmitDesc>(K);
+        SPK_CHECK_ARENA(ar);
         int tid_bits = 0; while ((1ll << tid_bits) < (long long)sp->n_contigs && tid_bits < 31) tid_bits++;
         int pos_bits = 1; while (pos_bits < 32 && (1ull << pos_bits) <= hsc->max_end) pos_bits++;
         size_t bytes = 0;
         if (pos_bits + tid_bits <= 32 && !getenv("SSB_SORT64")) {
-            uint32_t *key32 = arA.get<uint32_t>(K), *skey32 = arA.get<uint32_t>(K);
-            cub::DeviceRadixSort::SortPairs(NULL, bytes, key32, skey32, iota, perm, K, 0, pos_bits + tid_bits, sA);
-            void *tmp = arA.get<uint8_t>(bytes); SPK_CHECK_ARENA(arA);
-            SSB_LAUNCH_P(ctx, SSB_K_SPIKE_OTHER, pack_end_kernel, grid_for(K, 256), 256, 0, sA, k_end, K, pos_bits, key32, iota);
-            SSB_CUDA(ctx, cub::DeviceRadixSort::SortPairs(tmp, bytes, key32, skey32, iota, perm, K, 0, pos_bits + tid_bits, sA));   // stable: ties keep input order
-            SSB_LAUNCH_P(ctx, SSB_K_SPIKE_OTHER, unpack_end_kernel, grid_for(K, 256), 256, 0, sA, skey32, K, pos_bits, s_end);
+            uint32_t *key32 = ar.get<uint32_t>(K), *skey32 = ar.get<uint32_t>(K);
+            cub::DeviceRadixSort::SortPairs(NULL, bytes, key32, skey32, iota, perm, K, 0, pos_bits + tid_bits, s);
+            void *tmp = ar.get<uint8_t>(bytes); SPK_CHECK_ARENA(ar);
+            SSB_LAUNCH_P(ctx, SSB_K_SPIKE_OTHER, pack_end_kernel, grid_for(K, 256), 256, 0, s, k_end, K, pos_bits, key32, iota);
+            SSB_CUDA(ctx, cub::DeviceRadixSort::SortPairs(tmp, bytes, key32, skey32, iota, perm, K, 0, pos_bits + tid_bits, s));   // stable: ties keep input order
+            SSB_LAUNCH_P(ctx, SSB_K_SPIKE_OTHER, unpack_end_kernel, grid_for(K, 256), 256, 0, s, skey32, K, pos_bits, s_end);
         } else {
-            SSB_LAUNCH_P(ctx, SSB_K_SPIKE_OTHER, iota_kernel, grid_for(K, 256), 256, 0, sA, iota, K);
-            cub::DeviceRadixSort::SortPairs(NULL, bytes, k_end, s_end, iota, perm, K, 0, 32 + tid_bits + 1, sA);
-            void *tmp = arA.get<uint8_t>(bytes); SPK_CHECK_ARENA(arA);
-            SSB_CUDA(ctx, cub::DeviceRadixSort::SortPairs(tmp, bytes, k_end, s_end, iota, perm, K, 0, 32 + tid_bits + 1, sA));   // stable: ties keep input order
+            SSB_LAUNCH_P(ctx, SSB_K_SPIKE_OTHER, iota_kernel, grid_for(K, 256), 256, 0, s, iota, K);
+            cub::DeviceRadixSort::SortPairs(NULL, bytes, k_end, s_end, iota, perm, K, 0, 32 + tid_bits + 1, s);
+            void *tmp = ar.get<uint8_t>(bytes); SPK_CHECK_ARENA(ar);
+            SSB_CUDA(ctx, cub::DeviceRadixSort::SortPairs(tmp, bytes, k_end, s_end, iota, perm, K, 0, 32 + tid_bits + 1, s));   // stable: ties keep input order
         }
         ctx->launches += 8;
-        SSB_CUDA(ctx, cudaEventRecord(sp->ev_sort, sA));
-        SSB_LAUNCH_P(ctx, SSB_K_SPIKE_OTHER, outlen_kernel, grid_for(K, 256), 256, 0, sA, perm, s_end, k_desc, K, rg, olen, edesc, &dscA->n_owned);
-        if ((rc = scan_sum(arA, ctx, olen, out_off, K))) return rc;
-        SSB_LAUNCH(ctx, out_total_kernel, 1, 32, 0, sA, out_off, olen, K, &dscA->total_out);
-        SSB_LAUNCH_P(ctx, SSB_K_SPIKE_OTHER, ordoff_kernel, grid_for(K, 256), 256, 0, sA, perm, out_off, K, ord_off);
-        SSB_CUDA(ctx, cudaEventRecord(sp->ev_outoff, sA));
+        SSB_LAUNCH_P(ctx, SSB_K_SPIKE_OTHER, outlen_kernel, grid_for(K, 256), 256, 0, s, perm, s_end, k_desc, K, rg, olen, d_edesc, &dsc->n_owned);
+        if ((rc = scan_sum(ar, ctx, olen, out_off, K))) return rc;
+        SSB_LAUNCH(ctx, out_total_kernel, 1, 32, 0, s, out_off, olen, K, &dsc->total_out);
+        SSB_LAUNCH_P(ctx, SSB_K_SPIKE_OTHER, ordoff_kernel, grid_for(K, 256), 256, 0, s, perm, out_off, K, ord_off);
         if (out_cap < n + 1) {                 // the output may not fit: look before writing
-            if ((rc = publishA())) return rc;
-            if (hscA->total_out > out_cap) { snprintf(ctx->err, sizeof ctx->err, "spike: output needs %llu bytes, capacity %zu", (unsigned long long)hscA->total_out, out_cap); return SSB_E_ARG; }
+            if ((rc = publish())) return rc;
+            if (hsc->total_out > out_cap) { snprintf(ctx->err, sizeof ctx->err, "spike: output needs %llu bytes, capacity %zu", (unsigned long long)hsc->total_out, out_cap); return SSB_E_ARG; }
         }
-        d_edesc = edesc;
-    } else SSB_CUDA(ctx, cudaEventRecord(sp->ev_sort, sA));
-    // The copy of the text (DRAM bound) and the tallies are held back until the chain branch reaches its long issue-bound stretch
-    // (phase 1), so that they run beside it instead of slowing the short kernels before it down.
-    bool emit_launched = false;
-    auto launch_emit = [&]() -> int {
-        if (emit_launched) return SSB_OK;
-        emit_launched = true;
-        cudaStream_t se = sched == 1 ? sA : s;
-        if (K) {
-            if (se != sA) SSB_CUDA(ctx, cudaStreamWaitEvent(se, sp->ev_outoff, 0));
-            SSB_CUDA(ctx, cudaEventRecord(sp->ev_t[8], se));
-            const char *ev_ = getenv("SSB_EMIT_VARIANT"); const int v = ev_ ? atoi(ev_) : 0;
-            const int per_sm = (v >= 2 && v <= 8) ? v : (sched == 1 ? 3 : 8);   // resident emit blocks per SM (beside the chain branch: fewer)
-            if (v == 1) SSB_LAUNCH_P(ctx, SSB_K_SPIKE_EMIT, (emit_kernel<2, 4>), ctx->sm_count * 4, 256, 0, se, d_sam, n, d_edesc, out_off, K, d_out);
-            else SSB_LAUNCH_P(ctx, SSB_K_SPIKE_EMIT, (emit_kernel<1, 8>), ctx->sm_count * per_sm, 256, 0, se, d_sam, n, d_edesc, out_off, K, d_out);
-            SSB_CUDA(ctx, cudaEventRecord(sp->ev_t[9], se));
-        }
-        SSB_CUDA(ctx, cudaEventRecord(sp->ev_emit, se));
-        return SSB_OK;
-    };
+    }
 
     // ---------------------------------------------------------------- M: mates, coverage runs
     size_t R = 0; int64_t n_cov = 0;
@@ -632,54 +583,11 @@ int run_shard(ssb_spike *sp, const ShardPlan &pl, const uint8_t *d_sam, size_t n
         SSB_LAUNCH_P(ctx, SSB_K_SPIKE_OTHER, runs_kernel, grid_for(K, 256), 256, 0, s, k_start, ce, pm, rflag, rid, cbase, K, rg, runs);
         SSB_CUDA(ctx, cudaMemsetAsync(cum_e, 0, ((size_t)n_cov + 1) * sizeof(uint32_t), s));       // loci before the first read end
         SSB_LAUNCH_P(ctx, SSB_K_SPIKE_OTHER, cum_fill_kernel, grid_for(K, 256), 256, 0, s, k_start, K, runs, R, n_cov, cum_s);
-        SSB_CUDA(ctx, cudaStreamWaitEvent(s, sp->ev_sort, 0));                                     // the end-sorted keys come from the output branch
         SSB_LAUNCH_P(ctx, SSB_K_SPIKE_OTHER, cum_fill_kernel, grid_for(K, 256), 256, 0, s, s_end, K, runs, R, n_cov, cum_e);
         SSB_LAUNCH_P(ctx, SSB_K_SPIKE_OTHER, maxdepth_kernel, ctx->sm_count * 8, 256, 0, s, cum_s, cum_e, n_cov, &dsc->maxdepth);
     }
-    SSB_CUDA(ctx, cudaEventRecord(sp->ev_cover, s));
     SSB_CUDA(ctx, cudaEventRecord(sp->ev_t[3], s));
     dbg_mark("covered");
-
-    // ---------------------------------------------------------------- A: tallies of the non-target loci (no odd patch known yet)
-    unsigned long long *err64 = NULL; unsigned int *minus = NULL;
-    TallyArgs TA;
-    memset(&TA, 0, sizeof TA);
-    const bool use_list = exc_list && !no_list && n_list <= exc_cap;
-    auto tally_pass = [&](cudaStream_t st) -> int {
-        SSB_CUDA(ctx, cudaMemsetAsync(err64, 0, ((size_t)n_cov + 1) * sizeof(unsigned long long), st));
-        SSB_CUDA(ctx, cudaMemsetAsync(minus, 0, ((size_t)n_cov + 1) * sizeof(unsigned int), st));
-        if (use_list) {
-            if (n_list) SSB_LAUNCH_P(ctx, SSB_K_SPIKE_TALLY, tally_resolve_kernel, grid_for((size_t)n_list, 128), 128, 0, st, TA, exc_list, n_list, keep, kord);
-        } else {
-            KMeta *kmeta = (st == sA ? arA : ar).get<KMeta>(K); SPK_CHECK_ARENA(st == sA ? arA : ar);
-            SSB_LAUNCH_P(ctx, SSB_K_SPIKE_TALLY, kmeta_kernel, grid_for(K, 256), 256, 0, st, recs, k_rec, K, kmeta);
-            SSB_LAUNCH_P(ctx, SSB_K_SPIKE_TALLY, tally_fast_kernel, grid_for(K * 32, 128), 128, 0, st, TA, kmeta);
-        }
-        SSB_LAUNCH_P(ctx, SSB_K_SPIKE_TALLY, tally_kernel, grid_for(K, 128), 128, 0, st, TA);
-        return SSB_OK;
-    };
-    bool tally_launched = false;
-    auto launch_tally = [&]() -> int {
-        if (tally_launched) return SSB_OK;
-        tally_launched = true;
-        if (n_cov) {
-            int rc;
-            err64 = arA.get<unsigned long long>((size_t)n_cov + 1); minus = arA.get<unsigned int>((size_t)n_cov + 1);
-            SPK_CHECK_ARENA(arA);
-            TA.sam = d_sam; TA.recs = recs; TA.k_rec = k_rec; TA.k_start = k_start; TA.k_end = k_end; TA.k_hash = k_hash; TA.k_bits = k_bits; TA.K = K;
-            TA.nxt = nxt; TA.prv = prv; TA.cplx = cplx; TA.maxspan = h_maxspan; TA.runs = runs; TA.R = R;
-            TA.contig_seq = (const uint8_t *const *)sp->d_seq_ptrs; TA.contig_len = sp->d_lens; TA.err64 = err64; TA.minus = minus; TA.err = d_err;
-            TA.odd = d_odd; TA.n_odd = d_nodd; TA.odd_bloom = d_bloom; TA.listed_only = use_list ? 1 : 0; TA.rg = rg;
-            SSB_CUDA(ctx, cudaStreamWaitEvent(sA, sp->ev_cover, 0));
-            SSB_CUDA(ctx, cudaEventRecord(sp->ev_t[10], sA));
-            if ((rc = tally_pass(sA))) return rc;
-            SSB_CUDA(ctx, cudaEventRecord(sp->ev_t[11], sA));
-        }
-        SSB_CUDA(ctx, cudaEventRecord(sp->ev_tally, sA));
-        return SSB_OK;
-    };
-    // held: the output branch starts beside phase 1 (see launch_emit)
-    auto launch_output_branch = [&]() -> int { int rc; if ((rc = launch_emit())) return rc; return launch_tally(); };
 
     // ---------------------------------------------------------------- shards: who owns how many loci
     long long ord_base = 0, total_cov = n_cov;
@@ -938,7 +846,44 @@ int run_shard(ssb_spike *sp, const ShardPlan &pl, const uint8_t *d_sam, size_t n
     }
     SSB_CUDA(ctx, cudaEventRecord(sp->ev_t[5], s));
     dbg_mark("gathered");
-    { int rc; if ((rc = launch_output_branch())) return rc; }
+
+    // ---------------------------------------------------------------- emit
+    if (K) {
+        SSB_CUDA(ctx, cudaEventRecord(sp->ev_t[8], s));
+        SSB_LAUNCH_P(ctx, SSB_K_SPIKE_EMIT, emit_kernel, ctx->sm_count * 8, 256, 0, s, d_sam, n, d_edesc, out_off, K, d_out);
+        SSB_CUDA(ctx, cudaEventRecord(sp->ev_t[9], s));
+    }
+
+    // ---------------------------------------------------------------- tallies of the non-target loci (no odd patch known yet)
+    unsigned long long *err64 = NULL; unsigned int *minus = NULL;
+    TallyArgs TA;
+    memset(&TA, 0, sizeof TA);
+    const bool use_list = exc_list && !no_list && n_list <= exc_cap;
+    auto tally_pass = [&]() -> int {
+        SSB_CUDA(ctx, cudaMemsetAsync(err64, 0, ((size_t)n_cov + 1) * sizeof(unsigned long long), s));
+        SSB_CUDA(ctx, cudaMemsetAsync(minus, 0, ((size_t)n_cov + 1) * sizeof(unsigned int), s));
+        if (use_list) {
+            if (n_list) SSB_LAUNCH_P(ctx, SSB_K_SPIKE_TALLY, tally_resolve_kernel, grid_for((size_t)n_list, 128), 128, 0, s, TA, exc_list, n_list, keep, kord);
+        } else {
+            KMeta *kmeta = ar.get<KMeta>(K); SPK_CHECK_ARENA(ar);
+            SSB_LAUNCH_P(ctx, SSB_K_SPIKE_TALLY, kmeta_kernel, grid_for(K, 256), 256, 0, s, recs, k_rec, K, kmeta);
+            SSB_LAUNCH_P(ctx, SSB_K_SPIKE_TALLY, tally_fast_kernel, grid_for(K * 32, 128), 128, 0, s, TA, kmeta);
+        }
+        SSB_LAUNCH_P(ctx, SSB_K_SPIKE_TALLY, tally_kernel, grid_for(K, 128), 128, 0, s, TA);
+        return SSB_OK;
+    };
+    if (n_cov) {
+        int rc;
+        err64 = ar.get<unsigned long long>((size_t)n_cov + 1); minus = ar.get<unsigned int>((size_t)n_cov + 1);
+        SPK_CHECK_ARENA(ar);
+        TA.sam = d_sam; TA.recs = recs; TA.k_rec = k_rec; TA.k_start = k_start; TA.k_end = k_end; TA.k_hash = k_hash; TA.k_bits = k_bits; TA.K = K;
+        TA.nxt = nxt; TA.prv = prv; TA.cplx = cplx; TA.maxspan = h_maxspan; TA.runs = runs; TA.R = R;
+        TA.contig_seq = (const uint8_t *const *)sp->d_seq_ptrs; TA.contig_len = sp->d_lens; TA.err64 = err64; TA.minus = minus; TA.err = d_err;
+        TA.odd = d_odd; TA.n_odd = d_nodd; TA.odd_bloom = d_bloom; TA.listed_only = use_list ? 1 : 0; TA.rg = rg;
+        SSB_CUDA(ctx, cudaEventRecord(sp->ev_t[10], s));
+        if ((rc = tally_pass())) return rc;
+        SSB_CUDA(ctx, cudaEventRecord(sp->ev_t[11], s));
+    }
 
     // ---- shards: where in the stream does this shard begin (expected), and how sure is that
     double c_in = (double)k_in, v_in = 0;
@@ -1061,9 +1006,7 @@ int run_shard(ssb_spike *sp, const ShardPlan &pl, const uint8_t *d_sam, size_t n
             SSB_CUDA(ctx, cudaMemsetAsync(d_pool_used, 0, 8, s));
             SSB_CUDA(ctx, cudaMemsetAsync(d_lists, 0, (n_slices + SPARE) * (size_t)Rg * sizeof(BoundaryList), s));
             SSB_CUDA(ctx, cudaEventRecord(sp->ev_t[14], s));
-            auto p1k = phase1_kernel<P1_STAGES>;                 // SSB_P1_STAGES: conflicts resolved per walker step (measurement switch)
-            if (const char *e = getenv("SSB_P1_STAGES")) { const int v = atoi(e); p1k = v == 1 ? phase1_kernel<1> : v == 2 ? phase1_kernel<2> : v == 3 ? phase1_kernel<3> : v == 4 ? phase1_kernel<4> : v == 5 ? phase1_kernel<5> : phase1_kernel<6>; }
-            SSB_LAUNCH_P(ctx, SSB_K_SPIKE_CHAIN, p1k, (int)n_slices, P1_THREADS, P1_SMEM, s, A, Lc, d_groups, d_slices, kbuf, lobuf, wstride,
+            SSB_LAUNCH_P(ctx, SSB_K_SPIKE_CHAIN, phase1_kernel, (int)n_slices, P1_THREADS, P1_SMEM, s, A, Lc, d_groups, d_slices, kbuf, lobuf, wstride,
                          d_lists, Rg, pool_k, pool_lo, d_pool_used, pool_cap, d_flags, d_dbg, 0);
             SSB_CUDA(ctx, cudaEventRecord(sp->ev_t[15], s));
             SSB_LAUNCH_P(ctx, SSB_K_SPIKE_CHAIN, map_fill_kernel, (int)n_slices, 128, 0, s, d_groups, d_slices, d_lists, Rg, pool_k, pool_lo, kbuf, 0);     // group maps as flat tables (over the walker slots)
@@ -1128,7 +1071,7 @@ int run_shard(ssb_spike *sp, const ShardPlan &pl, const uint8_t *d_sam, size_t n
                     SSB_LAUNCH(ctx, copy_words_kernel, 1, 32, 0, s, (const uint32_t *)gd_, (uint32_t *)(d_groups + q), (unsigned int)(sizeof gd / 4));
                     SSB_LAUNCH(ctx, copy_words_kernel, 1, 32, 0, s, (const uint32_t *)sd_, (uint32_t *)(d_slices + n_slices + retry), (unsigned int)(sizeof sd / 4));
                     if ((rc = reset_state())) return rc;
-                    SSB_LAUNCH_P(ctx, SSB_K_SPIKE_CHAIN, p1k, 1, P1_THREADS, P1_SMEM, s, A, Lc, d_groups, d_slices, kbuf, lobuf, wstride,
+                    SSB_LAUNCH_P(ctx, SSB_K_SPIKE_CHAIN, phase1_kernel, 1, P1_THREADS, P1_SMEM, s, A, Lc, d_groups, d_slices, kbuf, lobuf, wstride,
                                  d_lists, Rg, pool_k, pool_lo, d_pool_used, pool_cap, d_flags, (unsigned long long *)NULL, (int)(n_slices + retry));
                     SSB_LAUNCH_P(ctx, SSB_K_SPIKE_CHAIN, map_fill_kernel, 1, 128, 0, s, d_groups, d_slices, d_lists, Rg, pool_k, pool_lo, kbuf, (int)(n_slices + retry));
                     n_retries++;
@@ -1204,9 +1147,7 @@ int run_shard(ssb_spike *sp, const ShardPlan &pl, const uint8_t *d_sam, size_t n
     stats->rng_k_in = (int64_t)k_in; stats->rng_k_out = (int64_t)k_out_final;
     stats->rng_draws = (int64_t)k_out_final;
 
-    // ---------------------------------------------------------------- join the output branch; patches
-    SSB_CUDA(ctx, cudaStreamWaitEvent(s, sp->ev_emit, 0));
-    SSB_CUDA(ctx, cudaStreamWaitEvent(s, sp->ev_tally, 0));
+    // ---------------------------------------------------------------- patches
     std::vector<FwdPatch> fwd_out, fwd_in;
     {
         int rc;
@@ -1256,7 +1197,7 @@ int run_shard(ssb_spike *sp, const ShardPlan &pl, const uint8_t *d_sam, size_t n
     // ---------------------------------------------------------------- SEQ_ERROR records
     if (n_cov) {
         int rc;
-        if (hsc->n_odd) { if ((rc = tally_pass(s))) return rc; }                                  // odd patches change bases later loci see: tally again with the list
+        if (hsc->n_odd) { if ((rc = tally_pass())) return rc; }                                 // odd patches change bases later loci see: tally again with the list
         if (H) SSB_LAUNCH_P(ctx, SSB_K_SPIKE_OTHER, tally_clear_hits_kernel, grid_for(H, 256), 256, 0, s, hits, H, err64);
         uint32_t *sflag = ar.get<uint32_t>((size_t)n_cov), *sidx = ar.get<uint32_t>((size_t)n_cov);
         SPK_CHECK_ARENA(ar);
@@ -1293,19 +1234,18 @@ int run_shard(ssb_spike *sp, const ShardPlan &pl, const uint8_t *d_sam, size_t n
             SSB_LAUNCH(ctx, copy_words_kernel, 64, 256, 0, s, (const uint32_t *)(d_res + r_lo), (uint32_t *)hr_dev, (unsigned int)(nb / 4));
         }
     }
-    { int rc; if ((rc = publish())) return rc; if ((rc = publishA())) return rc; }
+    { int rc; if ((rc = publish())) return rc; }
     SSB_CUDA(ctx, cudaStreamSynchronize(s));
-    SSB_CUDA(ctx, cudaStreamSynchronize(sA));
     if (hsc->err.code) return fail_dev("finish");
     if (T && d_res) {
         if (seq) for (size_t t = 0; t < T; t++) if (t < r_lo || t >= r_hi) { memset(&results[t], 0, sizeof results[t]); results[t].status = SSB_T_ELSEWHERE; results[t].at_tid = -1; results[t].at_pos = -1; results[t].rng_offset = -1; }
         if (r_hi > r_lo) memcpy(results + r_lo, sp->h_res, (r_hi - r_lo) * sizeof(ssb_target_result));
     }
-    *out_bytes = (size_t)hscA->total_out;
-    stats->out_bytes = (int64_t)hscA->total_out;
-    stats->alignmentCount = (int64_t)hscA->n_owned;                                       // every read is written exactly once, by the shard that owns its last base (:1275,:1365)
+    *out_bytes = (size_t)hsc->total_out;
+    stats->out_bytes = (int64_t)hsc->total_out;
+    stats->alignmentCount = (int64_t)hsc->n_owned;                                        // every read is written exactly once, by the shard that owns its last base (:1275,:1365)
     stats->maxDepth = (int64_t)hsc->maxdepth;
-    if (hscA->total_out > out_cap) { snprintf(ctx->err, sizeof ctx->err, "spike: output needs %llu bytes, capacity %zu", (unsigned long long)hscA->total_out, out_cap); return SSB_E_ARG; }
+    if (hsc->total_out > out_cap) { snprintf(ctx->err, sizeof ctx->err, "spike: output needs %llu bytes, capacity %zu", (unsigned long long)hsc->total_out, out_cap); return SSB_E_ARG; }
     if (hsc->maxdepth > (unsigned int)MAX_PILEUP) { snprintf(ctx->err, sizeof ctx->err, "spike: pileup depth %u exceeds MAX_PILEUP_SIZE", hsc->maxdepth); return SSB_E_DEPTH; }
     if (seq) {
         seq->k = k_out_final; seq->ord_base = ord_base + n_cov;

@@ -106,11 +106,11 @@ def test_parallel_chain_matches_serial(name, chunk, group, slice_, tmp_path, ctx
         assert st_p.chain_mode > 1, "expected the chunked chain to be used"
 
 
-@pytest.mark.parametrize("name,chunk,resident,stages", [("plain", 96, 3, 6), ("deep_lowvaf", 64, 2, 1), ("mask_n_ref", 128, 5, 3), ("two_contigs_window", 96, 1, 4)])
-def test_chain_geometry_is_chosen_to_fit_the_device(name, chunk, resident, stages, tmp_path, ctx, monkeypatch):
+@pytest.mark.parametrize("name,chunk,resident", [("plain", 96, 3), ("deep_lowvaf", 64, 2), ("mask_n_ref", 128, 5), ("two_contigs_window", 96, 1)])
+def test_chain_geometry_is_chosen_to_fit_the_device(name, chunk, resident, tmp_path, ctx, monkeypatch):
     """Phase 1 picks the group length and the slice width from the number of blocks the device holds at once (longer groups when the
     slices of the windows would not all be resident, then the narrowest slices that still fit).  With a "device" of a few blocks the
-    small inputs exercise what a shard far down the stream does at full size; the walker step runs with 1, 3, 4 and 6 stages.
+    small inputs exercise what a shard far down the stream does at full size.
     Same SAM, same per-target results and the same draw count as the one-warp serial chain and the reference."""
     prefix = sc.generate(name, str(tmp_path))
     want = sc.run_cli(sc.CHECKER, prefix, str(tmp_path / "ora"), cmdname="stochasticSpike")
@@ -124,7 +124,6 @@ def test_chain_geometry_is_chosen_to_fit_the_device(name, chunk, resident, stage
         monkeypatch.delenv("SSB_CHAIN_SERIAL")
         monkeypatch.setenv("SSB_CHAIN_CHUNK", str(chunk))
         monkeypatch.setenv("SSB_P1_RESIDENT", str(resident))
-        monkeypatch.setenv("SSB_P1_STAGES", str(stages))
         monkeypatch.setenv("SSB_SORT64", "1")              # and the 8-byte end-order keys (genomes whose keys do not fit 32 bits)
         out_p, res_p, st_p = s.run_host(body, targets, 434)
     assert hdr + out_s == want[2] and hdr + out_p == want[2]
