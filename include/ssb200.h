@@ -74,7 +74,7 @@ uint64_t ssb_kernel_launches(const ssb_ctx *ctx);
  * CUDA events on its own stream; ssb_profile_read() synchronises and returns the summed duration
  * and the number of launches of one kernel slot (and optionally resets them). */
 enum { SSB_PROF_TNC_SCAN = 0, SSB_PROF_TNC_FIXUP = 1, SSB_PROF_SPIKE_PARSE = 2, SSB_PROF_SPIKE_EMIT = 3,
-       SSB_PROF_SPIKE_CHAIN = 4, SSB_PROF_SPIKE_OTHER = 5, SSB_PROF_SPIKE_TALLY = 6 };
+       SSB_PROF_SPIKE_CHAIN = 4, SSB_PROF_SPIKE_OTHER = 5, SSB_PROF_SPIKE_TALLY = 6, SSB_PROF_TNC_INTERVALS = 7 };
 int  ssb_profile_enable(ssb_ctx *ctx, int on);
 int  ssb_profile_read(ssb_ctx *ctx, int slot, double *total_ms, uint64_t *launches, int reset);
 
@@ -133,8 +133,25 @@ int ssb_fasta_index(const uint8_t *fasta, size_t n, ssb_fasta_contig *out, const
 int ssb_tnc_count_bed_device(ssb_ctx *ctx, const uint8_t *d_fasta, size_t n, const ssb_fasta_contig *contigs, size_t n_contigs,
                              const ssb_bed_interval *intervals, size_t n_intervals, size_t first, size_t last, int64_t *d_counts64);
 
-/* The reference's 32-line stdout (tncCountsProfile.c:452-483): "CTX\t%ld\n", ctx + reverse
- * complement, fixed order.  Returns bytes written (excluding NUL) or SSB_E_ARG if cap is short. */
+/* Per-interval counts: adds the windows of each interval [first, last), on its own, to row (i - first) of d_rows
+ * (int64[(last - first) * 64], device, caller zeroes it; counts64 layout per row).  Row i is DEFINED as what
+ * tncCountsProfile.c:391-447 counts on the FASTA `bedtools getfasta` writes for interval i alone: one header line, then the
+ * interval's bases on one line.  That reduces to: a window counts at every position p in [start, end-2) where bases p, p+1
+ * and p+2 are all upper-case A/C/G/T; line terminators of the genome text are skipped through the index.  So rows do not
+ * depend on BED order, duplicates or overlaps, and they do NOT add up to ssb_tnc_count_bed_device's total: that one also
+ * counts the one straddling window the reference sees between consecutive kept intervals.  The genome text is read in
+ * place (no extracted FASTA).  d_fasta is 16-byte aligned, of any size (64-bit offsets throughout); contigs[] is its index
+ * (ssb_fasta_index).  Refusals as in ssb_tnc_count_bed_device: end < start -> SSB_E_ARG; an interval outside its contig, or
+ * an index that does not describe the file -> SSB_E_FORMAT.  Asynchronous except for the error check. */
+int ssb_tnc_count_intervals_device(ssb_ctx *ctx, const uint8_t *d_fasta, size_t n, const ssb_fasta_contig *contigs, size_t n_contigs,
+                                   const ssb_bed_interval *intervals, size_t n_intervals, size_t first, size_t last, int64_t *d_rows);
+
+/* The reference's fold of the 64 contexts into its 32 output lines (tncCountsProfile.c:452-483): context + reverse
+ * complement, in the order of its printf block. */
+void ssb_tnc_fold32(const int64_t counts64[64], int64_t out32[32]);
+
+/* The reference's 32-line stdout (tncCountsProfile.c:452-483): "CTX\t%ld\n", the 32 values of ssb_tnc_fold32, fixed
+ * order.  Returns bytes written (excluding NUL) or SSB_E_ARG if cap is short. */
 int ssb_tnc_format(const int64_t counts64[64], char *dst, size_t cap);
 
 /* ------------------------------------------------------------------------------------------

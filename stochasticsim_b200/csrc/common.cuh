@@ -29,7 +29,7 @@ struct ssb_ctx {
 
 // kernel slots for ssb_profile_read()
 enum { SSB_K_TNC_SCAN = 0, SSB_K_TNC_FIXUP = 1, SSB_K_SPIKE_PARSE = 2, SSB_K_SPIKE_EMIT = 3, SSB_K_SPIKE_CHAIN = 4,
-       SSB_K_SPIKE_OTHER = 5, SSB_K_SPIKE_TALLY = 6, SSB_K_SLOTS = 8 };
+       SSB_K_SPIKE_OTHER = 5, SSB_K_SPIKE_TALLY = 6, SSB_K_TNC_INTERVALS = 7, SSB_K_SLOTS = 8 };
 void ssb_prof_begin(ssb_ctx *ctx, int slot, cudaStream_t s);
 void ssb_prof_end(ssb_ctx *ctx, int slot, cudaStream_t s);
 

@@ -78,6 +78,14 @@ __device__ __forceinline__ uint32_t not_acgtnl(uint32_t w, uint32_t sy)
     const uint32_t e0 = __byte_perm(TLO, THI, sy), e1 = __byte_perm(TLO, THI, sy >> 16);
     return w ^ __byte_perm(e0, e1, 0x6420);
 }
+// bit k = the top bit of byte k (a byte flag mask as 4 bits)
+__device__ __forceinline__ uint32_t msb4(uint32_t f) { return (((f >> 7) * 0x00204081u) >> 21) & 0xFu; }
+// reference codes (A 0, C 1, G 2, T 3) of the four bytes of x, one per byte (meaningful where the byte is an upper-case base)
+__device__ __forceinline__ uint32_t ref_codes4(uint32_t x) { const uint32_t sy = (x >> 1) & 0x03030303u; return sy ^ ((sy >> 1) & 0x01010101u); }
+// per byte of (prev, cur) codes: the index 16 r[i-2] + 4 r[i-1] + r[i] of the window that ends at byte i of cur
+__device__ __forceinline__ uint32_t win_index4(uint32_t prev, uint32_t cur) { return cur + 4u * __funnelshift_r(prev, cur, 24) + 16u * __funnelshift_r(prev, cur, 16); }
+// 0x80 in every byte of w that is an upper-case A C G T
+__device__ __forceinline__ uint32_t base_flags(uint32_t w) { return zero_bytes_mask(not_acgtnl(w, symbols(w))) & (w << 1); }
 // four symbols [a,b,c,d] (one per byte, each 0..5) -> base-6 bin a + 6b + 36c + 216d: one integer dot product
 __device__ __forceinline__ uint32_t pack4(uint32_t z) { return __dp4a(z, 0xD8240601u, 0u); }
 constexpr int TNC_BINS = 1296;
@@ -186,24 +194,22 @@ tnc_scan_kernel(const uint8_t *__restrict__ b, size_t n, const TncDevState *__re
                 }
                 if (anyn) {
 #pragma unroll
-                    for (int j = 0; j < 4; j++) nlmask |= ((((nf[j] >> 7) * 0x00204081u) >> 21) & 0xFu) << (4 * j);
+                    for (int j = 0; j < 4; j++) nlmask |= msb4(nf[j]) << (4 * j);
                     if (!INTERIOR && p0 + TNC_BPT > n) nlmask &= (1u << (n - p0)) - 1u;
                 }
                 if (!anyb) nobase = true;
                 else {
                     // base flags of positions -2 .. 15 as a bit mask (bit i+2 <-> position i); a window ends where three in a row are set
-                    const uint32_t hz = zero_bytes_mask(not_acgtnl(hw, symbols(hw))) & (hw << 1);
-                    uint32_t bm = ((((hz >> 7) * 0x00204081u) >> 21) & 0xFu) >> 2;                   // positions -2, -1 -> bits 0, 1
+                    const uint32_t hz = base_flags(hw);
+                    uint32_t bm = msb4(hz) >> 2;                                                      // positions -2, -1 -> bits 0, 1
 #pragma unroll
-                    for (int j = 0; j < 4; j++) bm |= ((((bf[j] >> 7) * 0x00204081u) >> 21) & 0xFu) << (2 + 4 * j);
+                    for (int j = 0; j < 4; j++) bm |= msb4(bf[j]) << (2 + 4 * j);
                     uint32_t win = bm & (bm >> 1) & (bm >> 2);                                        // bit i: window ending at position i
                     if (!INTERIOR && p0 + TNC_BPT > n) win &= (1u << (n - p0)) - 1u;
                     if (win) {
                         // reference codes (A 0, C 1, G 2, T 3) of every byte, then per byte the index 16 r[i-2] + 4 r[i-1] + r[i] of the window that ends there
-                        auto codes = [](uint32_t x) { const uint32_t sy = (x >> 1) & 0x03030303u; return sy ^ ((sy >> 1) & 0x01010101u); };
-                        auto index = [](uint32_t prev, uint32_t cur) { return cur + 4u * __funnelshift_r(prev, cur, 24) + 16u * __funnelshift_r(prev, cur, 16); };
-                        const uint32_t rh = codes(hw), r0 = codes(w[0]), r1 = codes(w[1]), r2 = codes(w[2]), r3 = codes(w[3]);
-                        const uint32_t xw[4] = {index(rh, r0), index(r0, r1), index(r1, r2), index(r2, r3)};
+                        const uint32_t rh = ref_codes4(hw), r0 = ref_codes4(w[0]), r1 = ref_codes4(w[1]), r2 = ref_codes4(w[2]), r3 = ref_codes4(w[3]);
+                        const uint32_t xw[4] = {win_index4(rh, r0), win_index4(r0, r1), win_index4(r1, r2), win_index4(r2, r3)};
 #pragma unroll
                         for (int j = 0; j < 4; j++) {
                             uint32_t wj = (win >> (4 * j)) & 0xFu;
@@ -673,6 +679,13 @@ __global__ void bed_len_kernel(const ssb_bed_interval *__restrict__ iv, size_t f
     len[i] = k < 0 ? 0ull : (unsigned long long)(iv[k].end - iv[k].start) + 3ull;        // ">\n" + bases + "\n"
 }
 __device__ __forceinline__ size_t fasta_byte(const ssb_fasta_contig &c, int64_t p) { return (size_t)c.seq_off + (size_t)p + (size_t)(p / c.line_bases) * (size_t)(c.line_bytes - c.line_bases); }
+// the interval lies inside its contig
+__host__ __device__ inline bool bed_iv_ok(const ssb_bed_interval &v, const ssb_fasta_contig *contigs, size_t n_contigs)
+{
+    return v.contig >= 0 && (size_t)v.contig < n_contigs && v.start >= 0 && v.end >= v.start && v.end <= contigs[v.contig].len;
+}
+// a byte the index places at a base position cannot be a line end or a header: then the index does not describe this file
+__device__ __forceinline__ bool not_a_sequence_byte(uint8_t ch) { return ch == '\n' || ch == '>'; }
 // one warp per record
 __global__ void bed_gather_kernel(const uint8_t *__restrict__ fa, size_t n, const ssb_fasta_contig *__restrict__ contigs, size_t n_contigs, const ssb_bed_interval *__restrict__ iv,
                                   size_t first, size_t n_own, long long ctx_iv, const unsigned long long *__restrict__ off, uint8_t *__restrict__ out, unsigned int *__restrict__ bad)
@@ -683,14 +696,14 @@ __global__ void bed_gather_kernel(const uint8_t *__restrict__ fa, size_t n, cons
     const long long k = i == 0 ? ctx_iv : (long long)(first + i - 1);
     if (k < 0) return;
     const ssb_bed_interval v = iv[k];
-    if (v.contig < 0 || (size_t)v.contig >= n_contigs || v.start < 0 || v.end < v.start || v.end > contigs[v.contig].len) { if (lane == 0) atomicOr(bad, 1u); return; }
+    if (!bed_iv_ok(v, contigs, n_contigs)) { if (lane == 0) atomicOr(bad, 1u); return; }
     const ssb_fasta_contig c = contigs[v.contig];
     uint8_t *o = out + off[i];
     if (lane == 0) { o[0] = '>'; o[1] = '\n'; o[2 + (v.end - v.start)] = '\n'; }
     for (int64_t p = v.start + lane; p < v.end; p += 32) {
         const size_t b = fasta_byte(c, p);
         const uint8_t ch = b < n ? fa[b] : (uint8_t)'\n';
-        if (ch == '\n' || ch == '>') atomicOr(bad, 2u);                  // the index does not describe this file
+        if (not_a_sequence_byte(ch)) atomicOr(bad, 2u);
         o[2 + (p - v.start)] = ch;
     }
 }
@@ -701,7 +714,7 @@ __global__ void bed_context_kernel(const uint8_t *__restrict__ fa, size_t n, con
     const int lane = threadIdx.x;
     for (long long k = (long long)first - 1; k >= 0; k--) {
         const ssb_bed_interval v = iv[k];
-        if (v.contig < 0 || (size_t)v.contig >= n_contigs || v.start < 0 || v.end > contigs[v.contig].len) continue;
+        if (!bed_iv_ok(v, contigs, n_contigs)) continue;
         const ssb_fasta_contig c = contigs[v.contig];
         bool any = false;
         for (int64_t p0 = v.start; p0 < v.end && !any; p0 += 32) {
@@ -772,6 +785,186 @@ extern "C" int ssb_tnc_count_bed_device(ssb_ctx *ctx, const uint8_t *d_fasta, si
         SSB_LAUNCH(ctx, sub_counts_kernel, 1, 64, 0, s, (unsigned long long *)d_counts64, (const unsigned long long *)d_tmp);
     }
     SSB_CUDA(ctx, cudaStreamSynchronize(s));
+    return SSB_OK;
+}
+
+// ---- Per-interval counts ---------------------------------------------------------------------------------------------------------------
+// Row i = what the reference counts on the FASTA that holds interval i alone (a header line, the bases on one line).  For one line the
+// reference's rules reduce to: a window counts at every p in [start, end-2) where bases p, p+1, p+2 are all upper-case A/C/G/T.  So the
+// genome text is read in place through the index -- no extracted FASTA.
+//
+// Work: an item is (interval, segment of at most IV_T windows); an interval of 1 or 2 bases is one item without windows, so that its
+// bytes are checked against the index like any other.  Every warp of a persistent grid takes one contiguous range of the item list
+// (equal item counts; the host finds where each range starts).  Per item the warp stages the segment's bases plus the 2-base halo into
+// shared memory with the line terminators removed (aligned 4-byte loads, 128 bytes per warp step), then takes the windows four at a time
+// from SWAR codes as the generic path of tnc_scan_kernel does, counting into a lane-private 64-bin shared histogram (column = lane:
+// no atomics, no bank conflicts).  The histogram is flushed when the warp leaves an interval: with plain adds when the warp covered the
+// whole interval (every short interval), with 64 global atomics when the interval is split between warps (long intervals, whole-genome bins).
+namespace {
+constexpr int IV_T = 2048;                        // windows per item
+constexpr int IV_WARPS = 4;                       // warps per block: 4 x (8 KiB histogram + 2 KiB stage) of static shared memory
+constexpr int IV_STAGE_WORDS = (4 + IV_T + 2 + 3) / 4 + 1;   // a zero word, then the segment's IV_T + 2 bases, then zero fill
+
+struct IvTask { unsigned long long iv, item, count; };   // a warp's range: `count` items from item `item` of interval `iv`
+
+__host__ __device__ inline unsigned long long iv_items(int64_t len) { return len <= 0 ? 0ull : len <= 2 ? 1ull : (unsigned long long)(len - 2 + IV_T - 1) / IV_T; }
+
+// the warp's histogram is added to `row` (plain adds when this warp owns the whole row, atomics otherwise) and zeroed
+__device__ __forceinline__ void iv_flush(uint32_t *h, int lane, int64_t *row, bool whole)
+{
+    __syncwarp();
+    uint32_t t0 = 0, t1 = 0;
+#pragma unroll 8
+    for (int j = 0; j < 32; j++) {                       // lane takes bins lane and lane + 32; (j + lane) & 31 spreads the banks
+        const int c = (j + lane) & 31;
+        t0 += h[lane * 32 + c]; h[lane * 32 + c] = 0;
+        t1 += h[(lane + 32) * 32 + c]; h[(lane + 32) * 32 + c] = 0;
+    }
+    if (whole) { if (t0) row[lane] += t0; if (t1) row[lane + 32] += t1; }
+    else {
+        if (t0) atomicAdd((unsigned long long *)&row[lane], (unsigned long long)t0);
+        if (t1) atomicAdd((unsigned long long *)&row[lane + 32], (unsigned long long)t1);
+    }
+    __syncwarp();
+}
+
+__global__ void __launch_bounds__(IV_WARPS * 32)
+tnc_intervals_kernel(const uint8_t *__restrict__ fa, size_t n, const ssb_fasta_contig *__restrict__ contigs, const ssb_bed_interval *__restrict__ iv,
+                     const IvTask *__restrict__ tasks, size_t n_tasks, int64_t *__restrict__ rows, unsigned int *__restrict__ bad)
+{
+    __shared__ uint32_t hist[IV_WARPS][64 * 32];
+    __shared__ uint32_t stage[IV_WARPS][IV_STAGE_WORDS];
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const size_t gw = (size_t)blockIdx.x * IV_WARPS + wid;
+    if (gw >= n_tasks) return;
+    uint32_t *h = hist[wid], *st = stage[wid];
+    uint8_t *stb = reinterpret_cast<uint8_t *>(st) + 4;   // base j of the segment; st[0] stays 0 (no window ends before base 2)
+    for (int i = lane; i < 64 * 32; i += 32) h[i] = 0;
+    if (lane == 0) st[0] = 0;
+    const IvTask t = tasks[gw];
+    size_t i = (size_t)t.iv;
+    unsigned long long k = t.item, left = t.count;
+    bool whole = k == 0, counted = false;
+    while (left) {
+        const ssb_bed_interval v = iv[i];
+        const unsigned long long ni = iv_items(v.end - v.start);
+        if (ni == 0) { i++; continue; }
+        const ssb_fasta_contig c = contigs[v.contig];
+        const int64_t s = v.start + (int64_t)k * IV_T, e = min(s + IV_T + 2, v.end);
+        const uint32_t m = (uint32_t)(e - s);
+        const size_t tbs = fasta_byte(c, s), tbe = fasta_byte(c, e - 1);
+        if (tbe >= n) { if (lane == 0) atomicOr(bad, 2u); }
+        else {
+            // ---- stage bases [s, e) into stb[0, m): text byte a >= tbs sits in column (col0 + a - tbs) mod line_bytes of line
+            //      (col0 + a - tbs) / line_bytes, counted from s's line; it is a base when that column is < line_bases
+            __syncwarp();                                                 // the previous item's windows are counted
+            if (lane == 0) st[(m + 3) / 4] = 0;                           // zero the bytes after base m - 1 in its word
+            __syncwarp();
+            const uint32_t lb = c.line_bases, lbytes = c.line_bytes, col0 = (uint32_t)(s % lb);
+            const size_t a_end = tbe + 1;
+            bool badc = false;
+            for (size_t w0 = (tbs & ~(size_t)3) + 4 * lane; w0 < a_end; w0 += 4 * 128) {
+                uint32_t wd[4];
+#pragma unroll
+                for (int u = 0; u < 4; u++) { const size_t wa = w0 + 128 * u; wd[u] = wa < a_end ? ld_word(fa, n, wa) : 0u; }
+#pragma unroll
+                for (int u = 0; u < 4; u++) {
+                    const size_t wa = w0 + 128 * u;
+                    if (wa >= a_end) break;
+                    const uint32_t j0 = wa < tbs ? (uint32_t)(tbs - wa) : 0u;          // first byte of this word at or after s
+                    const uint32_t c0 = col0 + (uint32_t)(wa + j0 - tbs);
+                    uint32_t dl = c0 / lbytes, col = c0 - dl * lbytes;
+#pragma unroll
+                    for (uint32_t j = 0; j < 4; j++) {
+                        if (j < j0 || wa + j >= a_end) continue;
+                        const uint8_t ch = (uint8_t)(wd[u] >> (8 * j));
+                        const uint32_t d = dl * lb + col - col0;                    // (< m whenever the index is consistent)
+                        if (col < lb && d < m) { stb[d] = ch; badc |= not_a_sequence_byte(ch); }
+                        if (++col == lbytes) { col = 0; dl++; }
+                    }
+                }
+            }
+            if (badc) atomicOr(bad, 2u);
+            __syncwarp();
+            // ---- windows ending at bases 4(w-1) .. 4(w-1)+3, from the words w-1 and w of the stage
+            bool any = false;
+            for (uint32_t w = 1 + lane; w <= (m + 3) / 4; w += 32) {
+                const uint32_t prev = st[w - 1], cur = st[w];
+                const uint32_t bm = (msb4(base_flags(prev)) >> 2) | (msb4(base_flags(cur)) << 2);
+                uint32_t win = bm & (bm >> 1) & (bm >> 2) & 0xFu;
+                if (win) {
+                    const uint32_t x = win_index4(ref_codes4(prev), ref_codes4(cur));
+                    any = true;
+                    while (win) { const int b = __ffs(win) - 1; win &= win - 1; h[((x >> (8 * b)) & 63u) * 32 + lane]++; }
+                }
+            }
+            counted |= __any_sync(0xffffffffu, any);
+        }
+        left--;
+        if (++k == ni) {
+            if (counted) iv_flush(h, lane, rows + 64 * i, whole);
+            i++; k = 0; whole = true; counted = false;
+        }
+    }
+    if (counted) iv_flush(h, lane, rows + 64 * i, false);            // the range ends inside interval i: other warps share its row
+}
+} // namespace
+
+extern "C" int ssb_tnc_count_intervals_device(ssb_ctx *ctx, const uint8_t *d_fasta, size_t n, const ssb_fasta_contig *contigs, size_t n_contigs,
+                                              const ssb_bed_interval *intervals, size_t n_intervals, size_t first, size_t last, int64_t *d_rows)
+{
+    if (!ctx || (!d_fasta && n) || !d_rows || (n_contigs && !contigs) || (n_intervals && !intervals) || first > last || last > n_intervals) return SSB_E_ARG;
+    if (((uintptr_t)d_fasta & 15) != 0) return SSB_E_ARG;
+    if (first == last) return SSB_OK;
+    const size_t n_own = last - first;
+    const ssb_bed_interval *own = intervals + first;
+    unsigned long long total = 0;
+    bool outside = false;
+    for (size_t i = 0; i < n_own; i++) {
+        const ssb_bed_interval &v = own[i];
+        if (v.end < v.start) return SSB_E_ARG;
+        if (!bed_iv_ok(v, contigs, n_contigs)) { outside = true; continue; }
+        const ssb_fasta_contig &c = contigs[v.contig];
+        if (v.end > v.start && (c.line_bases == 0 || c.line_bytes < c.line_bases)) outside = true;   // no geometry to read it by
+        total += iv_items(v.end - v.start);
+    }
+    if (outside) { snprintf(ctx->err, sizeof ctx->err, "tnc/intervals: an interval lies outside its contig"); return SSB_E_FORMAT; }
+    if (total == 0) return SSB_OK;
+    SSB_CUDA(ctx, cudaSetDevice(ctx->device));
+    int per_sm = 0;
+    SSB_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, tnc_intervals_kernel, IV_WARPS * 32, 0));
+    unsigned long long n_warps = (unsigned long long)ctx->sm_count * (per_sm > 0 ? per_sm : 1) * IV_WARPS;
+    if (n_warps > total) n_warps = total;
+    // warp w takes items [total w / n_warps, total (w + 1) / n_warps)
+    std::vector<IvTask> tasks((size_t)n_warps);
+    unsigned long long before = 0, w = 0, lo = 0;
+    for (size_t i = 0; i < n_own && w < n_warps; i++) {
+        const unsigned long long ni = iv_items(own[i].end - own[i].start);
+        while (w < n_warps && lo < before + ni) {
+            const unsigned long long hi = (unsigned long long)((unsigned __int128)total * (w + 1) / n_warps);
+            tasks[w] = IvTask{i, lo - before, hi - lo};
+            lo = hi; w++;
+        }
+        before += ni;
+    }
+    // device copies of the index, this range's intervals and the ranges, in the context's scratch
+    auto up = [](size_t x) { return (x + 255) & ~(size_t)255; };
+    const size_t o_iv = up(n_contigs * sizeof *contigs), o_task = o_iv + up(n_own * sizeof *intervals), o_bad = o_task + up(tasks.size() * sizeof(IvTask));
+    int r = ssb_scratch_reserve(ctx, o_bad + 256);
+    if (r) return r;
+    uint8_t *base = (uint8_t *)ctx->scratch;
+    cudaStream_t st = ctx->stream;
+    SSB_CUDA(ctx, cudaMemcpyAsync(base, contigs, n_contigs * sizeof *contigs, cudaMemcpyHostToDevice, st));
+    SSB_CUDA(ctx, cudaMemcpyAsync(base + o_iv, own, n_own * sizeof *intervals, cudaMemcpyHostToDevice, st));
+    SSB_CUDA(ctx, cudaMemcpyAsync(base + o_task, tasks.data(), tasks.size() * sizeof(IvTask), cudaMemcpyHostToDevice, st));
+    SSB_CUDA(ctx, cudaMemsetAsync(base + o_bad, 0, sizeof(unsigned int), st));
+    const int grid = (int)((n_warps + IV_WARPS - 1) / IV_WARPS);
+    SSB_LAUNCH_P(ctx, SSB_K_TNC_INTERVALS, tnc_intervals_kernel, grid, IV_WARPS * 32, 0, st, d_fasta, n, (const ssb_fasta_contig *)base,
+                 (const ssb_bed_interval *)(base + o_iv), (const IvTask *)(base + o_task), tasks.size(), d_rows, (unsigned int *)(base + o_bad));
+    unsigned int h_bad = 0;
+    SSB_CUDA(ctx, cudaMemcpyAsync(&h_bad, base + o_bad, sizeof h_bad, cudaMemcpyDeviceToHost, st));
+    SSB_CUDA(ctx, cudaStreamSynchronize(st));
+    if (h_bad) { snprintf(ctx->err, sizeof ctx->err, "tnc/intervals: the FASTA index does not describe the file (line widths)"); return SSB_E_FORMAT; }
     return SSB_OK;
 }
 
@@ -881,15 +1074,24 @@ extern "C" int ssb_tnc_carry_after(const uint8_t *b, size_t n_, const ssb_tnc_ca
     return SSB_OK;
 }
 
+extern "C" void ssb_tnc_fold32(const int64_t counts64[64], int64_t out32[32])
+{
+    for (int i = 0; i < 32; i++) {
+        const char *s = OUT_ORDER[i];
+        const int fwd = 16 * ref_code(s[0]) + 4 * ref_code(s[1]) + ref_code(s[2]);
+        const int rev = 16 * (3 - ref_code(s[2])) + 4 * (3 - ref_code(s[1])) + (3 - ref_code(s[0]));
+        out32[i] = counts64[fwd] + counts64[rev];
+    }
+}
+
 extern "C" int ssb_tnc_format(const int64_t counts64[64], char *dst, size_t cap)
 {
     if (!counts64 || !dst) return SSB_E_ARG;
+    int64_t o[32];
+    ssb_tnc_fold32(counts64, o);
     size_t used = 0;
     for (int i = 0; i < 32; i++) {
-        const char *s = OUT_ORDER[i];
-        int fwd = 16 * ref_code(s[0]) + 4 * ref_code(s[1]) + ref_code(s[2]);
-        int rev = 16 * (3 - ref_code(s[2])) + 4 * (3 - ref_code(s[1])) + (3 - ref_code(s[0]));
-        int w = snprintf(dst + used, cap - used, "%s\t%ld\n", s, (long)(counts64[fwd] + counts64[rev]));
+        int w = snprintf(dst + used, cap - used, "%s\t%ld\n", OUT_ORDER[i], (long)o[i]);
         if (w < 0 || (size_t)w >= cap - used) return SSB_E_ARG;
         used += (size_t)w;
     }

@@ -4,6 +4,10 @@
  *   tncCountsProfile <target fasta>            (same argv, stdout and exit codes as the reference)
  *   tncCountsProfile <genome fasta> <bed>      (extension, BASELINE config 3: the counts the reference gives on the FASTA that
  *                                               `bedtools getfasta -fi <genome> -bed <bed>` would write, without writing it)
+ *   tncCountsProfile <genome fasta> <bed> --per-interval
+ *                                              (extension: one row per BED interval, in BED order -- "chrom start end" and the 32
+ *                                               counts the reference gives on the FASTA getfasta writes for that interval alone,
+ *                                               after a "#chrom start end ACA ... TTT" header line; tab separated)
  *
  * Replaces main() of tncCountsProfile.c:366-485.  This file stays in C and only does what a host
  * has to do -- open/map the file, hand byte ranges to the GPU(s), print the 32 lines.  All
@@ -12,7 +16,8 @@
  *
  * Environment (the reference reads none; these only select hardware):
  *   SSB_GPUS=N      spread the file over the first N GPUs by byte range (default 1); the per-GPU
- *                   count vectors are combined with ONE NCCL all-reduce of 64 int64.
+ *                   count vectors are combined with ONE NCCL all-reduce of 64 int64.  With a BED the
+ *                   intervals are split into N ranges instead; per interval each GPU writes its own rows.
  *   SSB_DEVICE=i    first device ordinal (default 0).
  */
 #include <stdio.h>
@@ -39,6 +44,7 @@ typedef struct {
     int rc;
     /* BED mode: the whole genome text goes to every GPU, the intervals [first, last) are this GPU's share */
     const ssb_fasta_contig *contigs; size_t n_contigs; const ssb_bed_interval *iv; size_t n_iv, first, last; size_t n_all;
+    int64_t *rows;     /* --per-interval: 64 counters per interval of [first, last) (host), instead of `counts` */
 } shard_t;
 
 static void *shard_main(void *arg)
@@ -46,12 +52,14 @@ static void *shard_main(void *arg)
     shard_t *s = (shard_t *)arg;
     if (!s->iv) { s->rc = ssb_tnc_count_host(s->ctx, s->base + s->off, s->len, &s->carry_in, NULL, s->counts); return NULL; }
     void *d_fa = NULL, *d_cnt = NULL;
+    const size_t cnt_bytes = s->rows ? (s->last - s->first) * 64 * sizeof(int64_t) : sizeof s->counts;
     s->rc = ssb_dev_alloc(s->ctx, s->n_all + 64, &d_fa);
-    if (!s->rc) s->rc = ssb_dev_alloc(s->ctx, sizeof s->counts, &d_cnt);
+    if (!s->rc) s->rc = ssb_dev_alloc(s->ctx, cnt_bytes, &d_cnt);
     if (!s->rc) s->rc = ssb_memcpy_h2d(s->ctx, d_fa, s->base, s->n_all);
-    if (!s->rc) s->rc = ssb_memset_dev(s->ctx, d_cnt, 0, sizeof s->counts);
-    if (!s->rc) s->rc = ssb_tnc_count_bed_device(s->ctx, (const uint8_t *)d_fa, s->n_all, s->contigs, s->n_contigs, s->iv, s->n_iv, s->first, s->last, (int64_t *)d_cnt);
-    if (!s->rc) s->rc = ssb_memcpy_d2h(s->ctx, s->counts, d_cnt, sizeof s->counts);
+    if (!s->rc) s->rc = ssb_memset_dev(s->ctx, d_cnt, 0, cnt_bytes);
+    if (!s->rc && s->rows) s->rc = ssb_tnc_count_intervals_device(s->ctx, (const uint8_t *)d_fa, s->n_all, s->contigs, s->n_contigs, s->iv, s->n_iv, s->first, s->last, (int64_t *)d_cnt);
+    else if (!s->rc) s->rc = ssb_tnc_count_bed_device(s->ctx, (const uint8_t *)d_fa, s->n_all, s->contigs, s->n_contigs, s->iv, s->n_iv, s->first, s->last, (int64_t *)d_cnt);
+    if (!s->rc) s->rc = ssb_memcpy_d2h(s->ctx, s->rows ? (void *)s->rows : (void *)s->counts, d_cnt, cnt_bytes);
     if (!s->rc) s->rc = ssb_sync(s->ctx);
     if (d_fa) ssb_dev_free(s->ctx, d_fa);
     if (d_cnt) ssb_dev_free(s->ctx, d_cnt);
@@ -118,15 +126,21 @@ int main(int argc, char **argv)
     if ((size_t)ngpu > n / 4096 + 1) ngpu = (int)(n / 4096 + 1);
     /* BED mode (second argument) */
     ssb_fasta_contig *contigs = NULL; ssb_bed_interval *iv = NULL; size_t n_contigs = 0, n_iv = 0;
+    const char **names = NULL; uint32_t *nlens = NULL;
+    int64_t *rows = NULL;                                     /* --per-interval: 64 counters per interval */
     if (argc > 2 && argv[2]) {
         int rc = ssb_fasta_index(data, n, NULL, NULL, NULL, 0, &n_contigs);
         if (rc) { fprintf(stderr, "tncCountsProfile: %s: a record's lines are not all as wide as its first one (%s)\n", argv[1], ssb_strerror(rc)); return 3; }
         contigs = malloc((n_contigs + 1) * sizeof *contigs);
-        const char **names = malloc((n_contigs + 1) * sizeof *names); uint32_t *nlens = malloc((n_contigs + 1) * sizeof *nlens);
+        names = malloc((n_contigs + 1) * sizeof *names); nlens = malloc((n_contigs + 1) * sizeof *nlens);
         ssb_fasta_index(data, n, contigs, names, nlens, n_contigs, &n_contigs);
         iv = load_bed(argv[2], names, nlens, n_contigs, &n_iv);
         if (!iv) exit(EXIT_FAILURE);
         if ((size_t)ngpu > n_iv / 64 + 1) ngpu = (int)(n_iv / 64 + 1);
+        if (argc > 3 && argv[3] && !strcmp(argv[3], "--per-interval")) {
+            rows = malloc((n_iv + 1) * 64 * sizeof *rows);
+            if (!rows) { fprintf(stderr, "tncCountsProfile: out of host memory for %zu rows\n", n_iv); return 3; }
+        }
     }
 
     shard_t sh[64]; ssb_ctx *ctxs[64];
@@ -137,7 +151,8 @@ int main(int argc, char **argv)
         sh[g].ctx = ctxs[g]; sh[g].base = data;
         sh[g].off = (n / (size_t)ngpu * (size_t)g) & ~(size_t)31;
         if (iv) { sh[g].iv = iv; sh[g].n_iv = n_iv; sh[g].contigs = contigs; sh[g].n_contigs = n_contigs; sh[g].n_all = n;
-                  sh[g].first = n_iv * (size_t)g / (size_t)ngpu; sh[g].last = n_iv * (size_t)(g + 1) / (size_t)ngpu; }
+                  sh[g].first = n_iv * (size_t)g / (size_t)ngpu; sh[g].last = n_iv * (size_t)(g + 1) / (size_t)ngpu;
+                  if (rows) sh[g].rows = rows + sh[g].first * 64; }
     }
     for (int g = 0; g < ngpu; g++) {
         sh[g].len = (g + 1 < ngpu ? sh[g + 1].off : n) - sh[g].off;
@@ -150,6 +165,25 @@ int main(int argc, char **argv)
     for (int g = 1; g < ngpu; g++) pthread_join(th[g], NULL);
     for (int g = 0; g < ngpu; g++)
         if (sh[g].rc) { fprintf(stderr, "tncCountsProfile: %s (%s)\n", ssb_strerror(sh[g].rc), ssb_last_error(ctxs[g])); return 3; }
+    if (rows) {
+        /* header: the 32 names in the order of the reference's output lines (as ssb_tnc_format prints them) */
+        char names32[4096]; int64_t zero[64] = {0};
+        const int nw = ssb_tnc_format(zero, names32, sizeof names32);
+        if (nw < 0) return 3;
+        printf("#chrom\tstart\tend");
+        for (char *p = names32; p < names32 + nw; p = strchr(p, '\n') + 1) printf("\t%.*s", (int)(strchr(p, '\t') - p), p);
+        printf("\n");
+        /* the GPUs wrote their ranges of rows side by side: print them in BED order */
+        for (size_t i = 0; i < n_iv; i++) {
+            int64_t o[32];
+            ssb_tnc_fold32(rows + i * 64, o);
+            printf("%.*s\t%lld\t%lld", (int)nlens[iv[i].contig], names[iv[i].contig], (long long)iv[i].start, (long long)iv[i].end);
+            for (int k = 0; k < 32; k++) printf("\t%lld", (long long)o[k]);
+            printf("\n");
+        }
+        for (int g = 0; g < ngpu; g++) ssb_ctx_destroy(ctxs[g]);
+        return 0;
+    }
 
     int64_t total[64];
     if (ngpu == 1) memcpy(total, sh[0].counts, sizeof total);

@@ -75,12 +75,8 @@ def fasta_index(data):
     return out
 
 
-def count_bed_device(ctx, d_ptr, n, index, intervals, d_counts, first=0, last=None):
-    """Adds the windows of BED intervals [first, last) (in the order given; (contig index, start, end)) to the 64 device counters."""
-    L = lib()
-    L.ssb_tnc_count_bed_device.restype = C.c_int
-    L.ssb_tnc_count_bed_device.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.POINTER(FastaContig), C.c_size_t, C.POINTER(BedInterval), C.c_size_t,
-                                           C.c_size_t, C.c_size_t, C.c_void_p]
+def _index_and_intervals(index, intervals):
+    """ctypes arrays of an index ([(name, FastaContig)]) and of intervals ((contig index, start, end) rows, or an int64 array of them)."""
     carr = (FastaContig * max(1, len(index)))(*[c for _, c in index])
     if isinstance(intervals, np.ndarray):                      # structured rows (contig, start, end) as int64 columns
         iv = (BedInterval * max(1, len(intervals)))()
@@ -91,8 +87,55 @@ def count_bed_device(ctx, d_ptr, n, index, intervals, d_counts, first=0, last=No
         C.memmove(iv, raw.ctypes.data, raw.nbytes)
     else:
         iv = (BedInterval * max(1, len(intervals)))(*[BedInterval(c, 0, a, b) for c, a, b in intervals])
+    return carr, iv
+
+
+_IV_ARGS = [C.c_void_p, C.c_void_p, C.c_size_t, C.POINTER(FastaContig), C.c_size_t, C.POINTER(BedInterval), C.c_size_t, C.c_size_t, C.c_size_t, C.c_void_p]
+
+
+def count_bed_device(ctx, d_ptr, n, index, intervals, d_counts, first=0, last=None):
+    """Adds the windows of BED intervals [first, last) (in the order given; (contig index, start, end)) to the 64 device counters."""
+    L = lib()
+    L.ssb_tnc_count_bed_device.restype = C.c_int
+    L.ssb_tnc_count_bed_device.argtypes = _IV_ARGS
+    carr, iv = _index_and_intervals(index, intervals)
     last = len(intervals) if last is None else last
     check(L.ssb_tnc_count_bed_device(ctx.handle, d_ptr, n, carr, len(index), iv, len(intervals), first, last, d_counts), ctx.handle)
+
+
+def count_intervals_device(ctx, d_ptr, n, index, intervals, d_rows, first=0, last=None):
+    """Adds the windows of each BED interval i in [first, last), on its own, to row i - first of the device int64 rows
+    d_rows[(last - first) * 64] (ssb_tnc_count_intervals_device: no straddling windows, so rows are independent of BED order)."""
+    L = lib()
+    L.ssb_tnc_count_intervals_device.restype = C.c_int
+    L.ssb_tnc_count_intervals_device.argtypes = _IV_ARGS
+    carr, iv = _index_and_intervals(index, intervals)
+    last = len(intervals) if last is None else last
+    check(L.ssb_tnc_count_intervals_device(ctx.handle, d_ptr, n, carr, len(index), iv, len(intervals), first, last, d_rows), ctx.handle)
+
+
+_fold_src = None
+
+
+def fold32(counts):
+    """(..., 64) context counts -> (..., 32): the reference's output lines (ssb_tnc_fold32: context + reverse complement, OUT_ORDER)."""
+    global _fold_src
+    if _fold_src is None:
+        # each output line is the sum of two contexts; read which from ssb_tnc_fold32 itself, one context at a time
+        L = lib()
+        L.ssb_tnc_fold32.restype = None
+        L.ssb_tnc_fold32.argtypes = [C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
+        src = [[] for _ in range(32)]
+        e, o = np.zeros(64, dtype=np.int64), np.zeros(32, dtype=np.int64)
+        for k in range(64):
+            e[:] = 0
+            e[k] = 1
+            L.ssb_tnc_fold32(e.ctypes.data_as(C.POINTER(C.c_int64)), o.ctypes.data_as(C.POINTER(C.c_int64)))
+            for j in np.flatnonzero(o):
+                src[j].append(k)
+        _fold_src = np.array(src, dtype=np.int64).T               # (2, 32)
+    c = np.asarray(counts, dtype=np.int64)
+    return c[..., _fold_src[0]] + c[..., _fold_src[1]]
 
 
 def format_counts(counts64):
