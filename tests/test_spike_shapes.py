@@ -51,7 +51,10 @@ INT_RE = re.compile(r"0|[1-9][0-9]*")
 def _envelope_errors(sam: bytes):
     """Lines outside what htslib prints back unchanged, and lines out of coordinate order."""
     text = sam.decode()
-    names = re.findall(r"^@SQ\tSN:(\S+)", text, re.M)
+    sq = re.findall(r"^@SQ\tSN:(\S+)", text, re.M)
+    names = {}
+    for tid, name in enumerate(sq):
+        names.setdefault(name, tid)                             # the first @SQ of a name is its tid (sam_hdr_name2tid)
     errs, last = [], (-1, -1)
     for k, line in enumerate(l for l in text.split("\n") if l and not l.startswith("@")):
         f = line.split("\t")
@@ -66,7 +69,7 @@ def _envelope_errors(sam: bytes):
         ok = ok and all(re.fullmatch(r"[A-Za-z][A-Za-z0-9]:(i:-?(0|[1-9][0-9]*)|Z:[ -~]*)", t) for t in f[11:])
         if not ok:
             errs.append("line %d outside the envelope: %s" % (k, line[:200]))
-        key = (names.index(f[2]) if f[2] in names else len(names), int(f[3]))
+        key = (names.get(f[2], len(sq)), int(f[3]))
         if key < last:
             errs.append("line %d out of order: %s" % (k, line[:200]))
         last = key
