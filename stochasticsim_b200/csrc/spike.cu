@@ -299,23 +299,31 @@ __global__ void ordoff_kernel(const uint32_t *__restrict__ perm, const unsigned 
     if (o < K) ord_off[perm[o]] = out_off[o];
 }
 
-// One warp per output line, 16 bytes per lane: destination-aligned 16-byte stores; the source bytes of a chunk lie in two
-// aligned 16-byte source words, shifted into place.  The shift is the same for the whole line (= for the whole warp), so the
-// word part of it is a four-way switch over statically indexed registers.  Two lines are in flight per warp.
-struct EmitJob { const uint8_t *src; uint8_t *dst; uint32_t len, head, nvec, mis, add_nl;
-                 __device__ __forceinline__ const uint4 *S() const { return reinterpret_cast<const uint4 *>(src + head - mis); }
-                 __device__ __forceinline__ uint4 *D() const { return reinterpret_cast<uint4 *>(dst + head); } };
+// Emit copies segments, not lines.  In a coordinate-sorted input the output order (tid, end, input index) leaves the input order
+// only near reads that end before the reads above them, so runs of consecutive output lines are runs of consecutive input lines:
+// one shifted memcpy each.  A warp takes EMIT_TASK consecutive output lines (one descriptor per lane, 32 at a time), cuts them
+// where a line does not continue its predecessor in the input, and copies every segment with the whole warp.  A segment that runs
+// on past the task's last line is cut there and continued by the next task; the two write byte-disjoint parts of the 16-byte
+// destination word they share.
+constexpr int EMIT_TASK = 32;        // output lines per warp task: a multiple of 32
+constexpr int EMIT_ROWS = 3;         // independent 16-byte loads per lane in flight per round
+constexpr int EMIT_BLOCKS = 4;       // resident blocks of 256 threads per SM (64 registers; the launch fills them once).  Four loads at
+                                     // 3 blocks gain 2 % on long segments and lose 12 % on short ones (DESIGN.md section 7)
 
-__device__ __forceinline__ EmitJob emit_job(const uint8_t *__restrict__ sam, const EmitDesc r, unsigned long long off, uint8_t *__restrict__ out)
+// A segment is copied with destination-aligned 16-byte stores; the source bytes of a destination word lie in two aligned 16-byte
+// source words, shifted into place.  The shift is the same for the whole segment (= for the whole warp), so the word part of it
+// is a four-way switch over statically indexed registers, taken once per segment.
+struct EmitJob { const uint8_t *src; uint8_t *dst; unsigned long long len, nvec; uint32_t head, mis, add_nl; };
+
+__device__ __forceinline__ EmitJob emit_job(const uint8_t *src, uint8_t *dst, unsigned long long len, uint32_t add_nl)
 {
     EmitJob j;
-    j.src = sam + r.src_off; j.dst = out + off; j.len = r.len; j.add_nl = r.add_nl;
-    uint32_t head = (uint32_t)((16 - ((uintptr_t)j.dst & 15)) & 15);
-    if (head > j.len) head = j.len;
+    j.src = src; j.dst = dst; j.len = len; j.add_nl = add_nl;
+    uint32_t head = (uint32_t)((16 - ((uintptr_t)dst & 15)) & 15);
+    if (head > len) head = (uint32_t)len;
     j.head = head;
-    j.nvec = (j.len - head) >> 4;
-    const uint8_t *s0 = j.src + head;
-    j.mis = (uint32_t)((uintptr_t)s0 & 15);
+    j.nvec = (len - head) >> 4;
+    j.mis = (uint32_t)((uintptr_t)(src + head) & 15);
     return j;
 }
 template <int WQ>
@@ -327,49 +335,107 @@ __device__ __forceinline__ uint4 emit_shift(const uint4 A, const uint4 B, uint32
     o.z = __funnelshift_r(W[WQ + 2], W[WQ + 3], sh); o.w = __funnelshift_r(W[WQ + 3], W[WQ + 4], sh);
     return o;
 }
-__device__ __forceinline__ void emit_load(const EmitJob &j, uint32_t i, const uint8_t *sam_end, uint4 &A, uint4 &B)
+// The destination words i < nvec.  Destination word i takes source words i and i + 1 (word i + 1 only when mis != 0; it always holds
+// a byte of the segment then, so no word beyond the input's last byte is read).  Each source word is loaded once: lane l's second
+// word is lane l + 1's first, and lane 31's is lane 0's word of the next row, which lane 0 loads one row past the round.
+template <int WQ>
+__device__ __forceinline__ void emit_rows(const EmitJob &j, int lane)
 {
-    const uint4 *S = j.S();
-    A = __ldg(S + i);
-    B = make_uint4(0, 0, 0, 0);
-    if (j.mis && reinterpret_cast<const uint8_t *>(S + i + 1) < sam_end) B = __ldg(S + i + 1);
-}
-__device__ __forceinline__ void emit_store(const EmitJob &j, uint32_t i, const uint4 A, const uint4 B)
-{
-    const uint32_t sh = (j.mis & 3u) * 8u;
-    uint4 o;
-    switch (j.mis >> 2) {
-    case 0: o = emit_shift<0>(A, B, sh); break;
-    case 1: o = emit_shift<1>(A, B, sh); break;
-    case 2: o = emit_shift<2>(A, B, sh); break;
-    default: o = emit_shift<3>(A, B, sh); break;
+    const uint4 *S = reinterpret_cast<const uint4 *>(j.src + j.head - j.mis);
+    uint4 *D = reinterpret_cast<uint4 *>(j.dst + j.head);
+    const uint32_t sh = (j.mis & 3u) * 8u, extra = j.mis ? 1u : 0u;
+    for (unsigned long long left = j.nvec; left; ) {
+        const uint32_t n = left < 32u * EMIT_ROWS ? (uint32_t)left : 32u * EMIT_ROWS;     // destination words of this round
+        uint4 A[EMIT_ROWS + 1];
+#pragma unroll
+        for (int u = 0; u <= EMIT_ROWS; u++) {
+            const uint32_t w = 32u * u + lane;
+            A[u] = make_uint4(0, 0, 0, 0);
+            if (w < n + extra && (u < EMIT_ROWS || lane == 0)) A[u] = __ldg(S + w);
+        }
+#pragma unroll
+        for (int u = 0; u < EMIT_ROWS; u++) {
+            const uint4 V = lane == 0 ? A[u + 1] : A[u];
+            uint4 B;
+            B.x = __shfl_sync(0xffffffffu, V.x, lane + 1); B.y = __shfl_sync(0xffffffffu, V.y, lane + 1);
+            B.z = __shfl_sync(0xffffffffu, V.z, lane + 1); B.w = __shfl_sync(0xffffffffu, V.w, lane + 1);
+            const uint32_t i = 32u * u + lane;
+            if (i < n) D[i] = emit_shift<WQ>(A[u], B, sh);
+        }
+        S += 32 * EMIT_ROWS; D += 32 * EMIT_ROWS; left -= n;
     }
-    j.D()[i] = o;
 }
 __device__ __forceinline__ void emit_edges(const EmitJob &j, int lane)
 {
     // < 16 bytes up to the first aligned destination address (lanes 0..15) and < 16 tail bytes (lanes 16..31) in one pass
-    const uint32_t done = j.head + (j.nvec << 4);
-    const uint32_t off = lane < 16 ? (uint32_t)lane : done + (uint32_t)lane - 16u;
+    const unsigned long long done = j.head + (j.nvec << 4);
+    const unsigned long long off = lane < 16 ? (unsigned long long)lane : done + (unsigned long long)lane - 16u;
     const bool on = lane < 16 ? (uint32_t)lane < j.head : off < j.len;
     if (on) j.dst[off] = j.src[off];
     if (lane == 0 && j.add_nl) j.dst[j.len] = '\n';
 }
+// source bytes [s0, e0) to output offset d0, then a newline if `nl` (warp-uniform arguments)
+__device__ __forceinline__ void emit_segment(const uint8_t *sam, uint8_t *out, unsigned long long s0, unsigned long long e0,
+                                             unsigned long long d0, uint32_t nl, int lane)
+{
+    if (e0 == s0) return;                                   // lines another shard writes, lanes past the last line
+    const EmitJob j = emit_job(sam + s0, out + d0, e0 - s0, nl);
+    switch (j.mis >> 2) {
+    case 0: emit_rows<0>(j, lane); break;
+    case 1: emit_rows<1>(j, lane); break;
+    case 2: emit_rows<2>(j, lane); break;
+    default: emit_rows<3>(j, lane); break;
+    }
+    emit_edges(j, lane);
+}
 
-// one output line per warp
-__global__ void __launch_bounds__(256, 8)
-emit_kernel(const uint8_t *__restrict__ sam, size_t n_sam, const EmitDesc *__restrict__ desc, const unsigned long long *__restrict__ out_off, size_t K,
+__global__ void __launch_bounds__(256, EMIT_BLOCKS)
+emit_kernel(const uint8_t *__restrict__ sam, const EmitDesc *__restrict__ desc, const unsigned long long *__restrict__ out_off, size_t K,
             uint8_t *__restrict__ out)
 {
     const int lane = threadIdx.x & 31;
     const size_t warps = ((size_t)gridDim.x * blockDim.x) >> 5;
-    const uint8_t *sam_end = sam + n_sam;
-    for (size_t o = (((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5); o < K; o += warps) {
-        const EmitJob j = emit_job(sam, desc[o], out_off[o], out);
-        uint4 A, B;
-        if ((uint32_t)lane < j.nvec) { emit_load(j, lane, sam_end, A, B); emit_store(j, lane, A, B); }
-        for (uint32_t i = lane + 32; i < j.nvec; i += 32) { emit_load(j, i, sam_end, A, B); emit_store(j, i, A, B); }
-        emit_edges(j, lane);
+    const size_t tasks = (K + EMIT_TASK - 1) / EMIT_TASK;
+    for (size_t t = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; t < tasks; t += warps) {
+        // the open segment: source bytes [s0, e0) go to output offset d0, a newline follows if nl0
+        unsigned long long s0 = 0, e0 = 0, d0 = 0; uint32_t nl0 = 0;
+        unsigned long long prev_end = 0; bool prev_open = false;          // the line before lane 0's
+#pragma unroll 1
+        for (int c = 0; c < EMIT_TASK; c += 32) {
+            const size_t o = t * EMIT_TASK + c + lane;
+            EmitDesc d; d.src_off = 0; d.len = 0; d.add_nl = 0;
+            unsigned long long off = 0;
+            if (o < K) { d = desc[o]; off = out_off[o]; }
+            const unsigned long long end = d.src_off + d.len;
+            // a line continues its predecessor when it starts where that one ends in the input, neither is empty (a line another
+            // shard writes has len 0) and no newline is added in between (the output offsets of the two are then consecutive too)
+            const bool open = d.len > 0 && !d.add_nl;
+            unsigned long long pe = __shfl_up_sync(0xffffffffu, end, 1);
+            bool po = __shfl_up_sync(0xffffffffu, open, 1);
+            if (lane == 0) { pe = prev_end; po = prev_open; }
+            const bool cont = po && d.len > 0 && d.src_off == pe;
+            // bit k < 32: lane k starts a segment; bit 32: the task ends after this chunk.  Each of them closes the open segment.
+            unsigned long long ev = __ballot_sync(0xffffffffu, !cont);
+            if (c + 32 == EMIT_TASK) ev |= 1ull << 32;
+            prev_end = __shfl_sync(0xffffffffu, end, 31);
+            prev_open = __shfl_sync(0xffffffffu, open, 31);
+            if (!(ev & 1u)) {                                               // lanes before the first start extend the open segment
+                const int l = (uint32_t)ev ? __ffs((uint32_t)ev) - 2 : 31;
+                e0 = __shfl_sync(0xffffffffu, end, l);
+                nl0 = __shfl_sync(0xffffffffu, d.add_nl, l);
+            }
+            while (ev) {
+                const int f = __ffsll(ev) - 1;
+                ev &= ev - 1;
+                emit_segment(sam, out, s0, e0, d0, nl0, lane);
+                if (f == 32) break;
+                const int l = (uint32_t)ev ? __ffs((uint32_t)ev) - 2 : 31;   // the segment opened at lane f ends at lane l (or runs on)
+                s0 = __shfl_sync(0xffffffffu, d.src_off, f);
+                d0 = __shfl_sync(0xffffffffu, off, f);
+                e0 = __shfl_sync(0xffffffffu, end, l);
+                nl0 = __shfl_sync(0xffffffffu, d.add_nl, l);
+            }
+        }
     }
 }
 

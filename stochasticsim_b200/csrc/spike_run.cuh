@@ -850,7 +850,7 @@ int run_shard(ssb_spike *sp, const ShardPlan &pl, const uint8_t *d_sam, size_t n
     // ---------------------------------------------------------------- emit
     if (K) {
         SSB_CUDA(ctx, cudaEventRecord(sp->ev_t[8], s));
-        SSB_LAUNCH_P(ctx, SSB_K_SPIKE_EMIT, emit_kernel, ctx->sm_count * 8, 256, 0, s, d_sam, n, d_edesc, out_off, K, d_out);
+        SSB_LAUNCH_P(ctx, SSB_K_SPIKE_EMIT, emit_kernel, ctx->sm_count * EMIT_BLOCKS, 256, 0, s, d_sam, d_edesc, out_off, K, d_out);
         SSB_CUDA(ctx, cudaEventRecord(sp->ev_t[9], s));
     }
 
