@@ -805,7 +805,7 @@ struct TallyArgs {
     const CovRun *runs; size_t R; const uint8_t *const *contig_seq; const int64_t *contig_len;
     unsigned long long *err64; unsigned int *minus; DevErr *err;
     const OddPatch *odd; const unsigned int *n_odd; const unsigned long long *odd_bloom;
-    int listed_only;          // 1: the tokeniser's exception list is in use; fast reads it did not cover take the generic kernel
+    int listed_only;          // 1: tally_resolve_kernel settles the reads the tokeniser's exception list covers; 0: tally_kernel takes every read
     Range rg;                 // loci outside the shard's range belong to another shard's tallies
 };
 
@@ -843,133 +843,19 @@ __device__ __forceinline__ void tally_add(const TallyArgs &A, int64_t g, int con
     if (contrib >= 2) atomicAdd(&A.err64[g], 1ull << (16 * (contrib - 2)));
 }
 
-// A read takes the fast tally when every query base aligns 1:1 to the reference (CIGAR of M/=/X only), the only reads
-// that share its QNAME inside its span are its direct neighbours in the mate chain and are just as simple, and no odd
-// patch touched any of them.
-__device__ __forceinline__ bool tally_simple_read(const TallyArgs &A, size_t o, unsigned int n_odd, unsigned long long bloom)
+// A read is settled from the tokeniser's exception list iff every query base of it aligns 1:1 to the reference (CIGAR of
+// M/=/X only), the tokeniser listed its exceptional bases, no odd patch touched it, the only reads that share its QNAME
+// inside its span are its direct neighbours in the mate chain, and the same holds for those neighbours (a plain base only
+// changes its contribution when a neighbour's base over the same position is exceptional, and that entry is what triggers
+// the re-evaluation).  Every other read is self-contained work of tally_kernel.
+__device__ __forceinline__ bool tally_is_listed(const TallyArgs &A, size_t o, unsigned int n_odd, unsigned long long bloom)
 {
-    if (!(A.k_bits[o] & REC_SIMPLE) || A.cplx[o]) return false;
-    if (n_odd && (bloom & odd_bit((uint32_t)o))) return false;
-    return true;
-}
-__device__ __forceinline__ bool tally_is_fast(const TallyArgs &A, size_t o, const SamRec &r, unsigned int n_odd, unsigned long long bloom)
-{
-    if (!tally_simple_read(A, o, n_odd, bloom)) return false;
-    const uint32_t p = A.prv[o], q = A.nxt[o] & ~MATE_MORE;
-    if (p != PRV_NONE && !tally_simple_read(A, p, n_odd, bloom)) return false;
-    if (q != NO_MATE && !tally_simple_read(A, q, n_odd, bloom)) return false;
-    (void)r;
-    return true;
-}
-
-// List mode: a read is settled from the tokeniser's exception list iff it is fast-eligible, the tokeniser listed its own
-// exceptional bases, and it listed those of its mate-chain neighbours too (a plain base only changes its contribution when a
-// neighbour's base over the same position is exceptional, and that entry is what triggers the re-evaluation).  Every other
-// read is self-contained work of tally_kernel.
-__device__ __forceinline__ bool tally_is_listed(const TallyArgs &A, size_t o, const SamRec &r, unsigned int n_odd, unsigned long long bloom)
-{
-    if (!(A.k_bits[o] & REC_EXC_DONE) || !tally_is_fast(A, o, r, n_odd, bloom)) return false;
-    const uint32_t p = A.prv[o], q = A.nxt[o] & ~MATE_MORE;
-    if (p != PRV_NONE && !(A.k_bits[p] & REC_EXC_DONE)) return false;
-    if (q != NO_MATE && !(A.k_bits[q] & REC_EXC_DONE)) return false;
-    return true;
-}
-
-__device__ __forceinline__ uint32_t ldg_u32_unaligned(const uint8_t *p)
-{
-    const uint32_t a = (uint32_t)((uintptr_t)p & 3u);
-    const uint32_t *q = reinterpret_cast<const uint32_t *>(p - a);
-    return __funnelshift_r(__ldg(q), __ldg(q + 1), a * 8);
-}
-
-// 0x80 flags of the bytes of a simple read that are not plain "reference base with BQ > 0" at query offset w..w+3
-__device__ __forceinline__ uint32_t exc_word(const uint8_t *seq, const uint8_t *qual, bool qstar, uint32_t w, uint32_t refw)
-{
-    const uint32_t sq = ldg_u32_unaligned(seq + w);
-    const uint32_t ql = qstar ? 0x7e7e7e7eu : ldg_u32_unaligned(qual + w);
-    // a read N counts nothing, also where it equals a reference N (reads through the N runs of a real reference)
-    return (~samparse::zero_bytes(sq ^ refw) | samparse::zero_bytes(sq ^ 0x4E4E4E4Eu) | samparse::zero_bytes(ql ^ 0x21212121u)) & 0x80808080u;
-}
-
-// the rare path of the fast tally: one exceptional base of read o at reference position x, evaluated exactly
-__device__ __noinline__ void tally_exceptional_base(const TallyArgs &A, uint32_t o, int32_t x, int64_t g)
-{
-    const SamRec &r = A.recs[A.k_rec[o]];
-    ReadView mem[3]; int n = 0, self = 0;
-    const uint32_t p = A.prv[o], q = A.nxt[o] & ~MATE_MORE;
-    if (p != PRV_NONE && (uint32_t)A.k_end[p] > (uint32_t)r.pos) mem[n++] = view_of(A.sam, A.recs[A.k_rec[p]], p, NULL, 0, 0);
-    self = n; mem[n++] = view_of(A.sam, r, o, NULL, 0, 0);
-    if (q != NO_MATE) mem[n++] = view_of(A.sam, A.recs[A.k_rec[q]], q, NULL, 0, 0);
-    ReadView cov[3]; int nc = 0, sc = 0;
-    for (int m = 0; m < n; m++) if (mem[m].pos <= x && x < mem[m].end) { if (m == self) sc = nc; cov[nc++] = mem[m]; }
-    const uint8_t F = A.contig_seq[r.tid][x];
-    tally_add(A, g, chain_contribution(cov, nc, sc, x, F));
-}
-
-// Compact per-read metadata for the fast tally (one 32-byte load instead of a chain of dependent loads)
-struct __align__(16) KMeta { unsigned long long line_off; uint32_t seq_off, qual_off, l_seq; int32_t pos, end; uint32_t tid_bits; };
-static_assert(sizeof(KMeta) == 32, "KMeta layout");
-
-__global__ void kmeta_kernel(const SamRec *__restrict__ recs, const uint32_t *__restrict__ k_rec, size_t K, KMeta *__restrict__ km)
-{
-    size_t o = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (o >= K) return;
-    const SamRec &r = recs[k_rec[o]];
-    KMeta m; m.line_off = r.line_off; m.seq_off = r.seq_off; m.qual_off = r.qual_off; m.l_seq = r.l_seq; m.pos = r.pos; m.end = r.end;
-    m.tid_bits = ((uint32_t)r.tid << 8) | r.bits;
-    km[o] = m;
-}
-
-// One warp per read: SEQ, QUAL and the reference compared four bytes per lane; only bytes that differ from the
-// reference or have BQ 0 -- in this read or in an overlapping mate -- are evaluated one by one.
-__global__ void __launch_bounds__(128, 8)
-tally_fast_kernel(TallyArgs A, const KMeta *__restrict__ km)
-{
-    const int lane = threadIdx.x & 31;
-    const size_t o = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    if (o >= A.K) return;
-    const unsigned int n_odd = *A.n_odd; const unsigned long long bloom = *A.odd_bloom;
-    const KMeta me = km[o];
-    const uint32_t p = A.prv[o], q = A.nxt[o] & ~MATE_MORE;
-    auto simple_ok = [&](uint32_t idx, uint32_t tid_bits) {
-        return (tid_bits & REC_SIMPLE) && !A.cplx[idx] && !(n_odd && (bloom & odd_bit(idx)));
+    auto listed = [&](size_t i) {
+        return (A.k_bits[i] & REC_EXC_DONE) && (A.k_bits[i] & REC_SIMPLE) && !A.cplx[i] && !(n_odd && (bloom & odd_bit((uint32_t)i)));
     };
-    if (!simple_ok((uint32_t)o, me.tid_bits)) return;
-    KMeta mp, mq; mp.pos = 0; mp.end = 0; mq.pos = 0; mq.end = 0;
-    bool hp = false, hq = false;
-    if (p != PRV_NONE) { mp = km[p]; if (!simple_ok(p, mp.tid_bits)) return; hp = mp.end > me.pos; }
-    if (q != NO_MATE) { mq = km[q]; if (!simple_ok(q, mq.tid_bits)) return; hq = true; }
-    const int tid = (int)(me.tid_bits >> 8);
-    const uint8_t *ref = A.contig_seq[tid];
-    if (!ref || (int64_t)me.end > A.contig_len[tid]) { if (lane == 0) set_err(A.err, SSB_E_REF, me.line_off); return; }
-    size_t ri; { size_t lo = 0, hi = A.R; while (hi - lo > 1) { size_t mid = (lo + hi) >> 1;
-                   bool le = A.runs[mid].tid < tid || (A.runs[mid].tid == tid && A.runs[mid].start <= me.pos); if (le) lo = mid; else hi = mid; } ri = lo; }
-    const int64_t gbase = A.runs[ri].base - A.runs[ri].start + me.pos;    // covered ordinal of query offset 0
-    int64_t xl, xh; owned_span(A.rg, tid, xl, xh);
-    const uint8_t *seq = A.sam + me.line_off + me.seq_off, *qual = A.sam + me.line_off + me.qual_off, *rf = ref + me.pos;
-    const bool qstar = (me.tid_bits & REC_QUALSTAR) != 0;
-    const uint32_t L = me.l_seq;
-    for (uint32_t w = lane * 4; w < L; w += 128) {
-        const uint32_t rw = ldg_u32_unaligned(rf + w);
-        uint32_t exc = exc_word(seq, qual, qstar, w, rw);
-        const int32_t x0 = me.pos + (int32_t)w;
-        if (hp && !(x0 + 3 < mp.pos || x0 >= mp.end)) {
-            if (x0 >= mp.pos && x0 + 4 <= mp.end)
-                exc |= exc_word(A.sam + mp.line_off + mp.seq_off, A.sam + mp.line_off + mp.qual_off, (mp.tid_bits & REC_QUALSTAR) != 0, (uint32_t)(x0 - mp.pos), rw);
-            else exc = 0x80808080u;                                    // the mate starts or ends inside this word: look at every byte
-        }
-        if (hq && !(x0 + 3 < mq.pos || x0 >= mq.end)) {
-            if (x0 >= mq.pos && x0 + 4 <= mq.end)
-                exc |= exc_word(A.sam + mq.line_off + mq.seq_off, A.sam + mq.line_off + mq.qual_off, (mq.tid_bits & REC_QUALSTAR) != 0, (uint32_t)(x0 - mq.pos), rw);
-            else exc = 0x80808080u;
-        }
-        const uint32_t rem = L - w;
-        if (rem < 4) exc &= (1u << (8 * rem)) - 1u;
-        while (exc) {
-            const int k = (__ffs(exc) - 1) >> 3; exc &= exc - 1;
-            if (x0 + k >= xl && x0 + k < xh) tally_exceptional_base(A, (uint32_t)o, x0 + k, gbase + w + k);
-        }
-    }
+    if (!listed(o)) return false;
+    const uint32_t p = A.prv[o], q = A.nxt[o] & ~MATE_MORE;
+    return (p == PRV_NONE || listed(p)) && (q == NO_MATE || listed(q));
 }
 
 // One thread per exceptional base listed by the tokeniser: the base itself, and any mate lying over the same position
@@ -986,7 +872,7 @@ tally_resolve_kernel(TallyArgs A, const unsigned long long *__restrict__ list, u
     const uint32_t o = kord[line];
     const SamRec &r = A.recs[A.k_rec[o]];
     const unsigned int n_odd = *A.n_odd; const unsigned long long bloom = *A.odd_bloom;
-    const bool own = tally_is_listed(A, o, r, n_odd, bloom);           // else the read itself is tally_kernel's work
+    const bool own = tally_is_listed(A, o, n_odd, bloom);              // else the read itself is tally_kernel's work
     const int32_t x = r.pos + (int32_t)(e & 0xffff);
     { int64_t xl, xh; owned_span(A.rg, r.tid, xl, xh); if (x < xl || x >= xh) return; }
     size_t ri; { size_t lo = 0, hi = A.R; while (hi - lo > 1) { size_t mid = (lo + hi) >> 1;
@@ -1008,7 +894,7 @@ tally_resolve_kernel(TallyArgs A, const unsigned long long *__restrict__ list, u
         uint8_t b; int bq; bool sk;
         base_at(cov[m], x, b, bq, sk);
         // a plain base of a list-settled neighbour has no entry of its own: it matters only if it was marked handled here
-        if (b == F && b != 'N' && bq != 0 && tally_is_listed(A, cord[m], A.recs[A.k_rec[cord[m]]], n_odd, bloom)) tally_add(A, g, chain_contribution(cov, nc, m, x, F));
+        if (b == F && b != 'N' && bq != 0 && tally_is_listed(A, cord[m], n_odd, bloom)) tally_add(A, g, chain_contribution(cov, nc, m, x, F));
     }
 }
 
@@ -1019,7 +905,7 @@ tally_kernel(TallyArgs A)
     if (o >= A.K) return;
     const SamRec &r = A.recs[A.k_rec[o]];
     const unsigned int n_odd = *A.n_odd; const unsigned long long bloom = *A.odd_bloom;
-    if (A.listed_only ? tally_is_listed(A, o, r, n_odd, bloom) : tally_is_fast(A, o, r, n_odd, bloom)) return;   // settled by tally_resolve_kernel / tally_fast_kernel
+    if (A.listed_only && tally_is_listed(A, o, n_odd, bloom)) return;       // settled by tally_resolve_kernel
     const ReadView me = view_of(A.sam, r, (uint32_t)o, A.odd, n_odd, bloom);
     const int tid = r.tid;
     const uint8_t *ref = A.contig_seq[tid];

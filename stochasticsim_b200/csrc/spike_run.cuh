@@ -858,17 +858,11 @@ int run_shard(ssb_spike *sp, const ShardPlan &pl, const uint8_t *d_sam, size_t n
     unsigned long long *err64 = NULL; unsigned int *minus = NULL;
     TallyArgs TA;
     memset(&TA, 0, sizeof TA);
-    const bool use_list = exc_list && !no_list && n_list <= exc_cap;
+    const bool use_list = exc_list && !no_list && n_list <= exc_cap;           // else (overflow, SSB_NO_EXC_LIST) tally_kernel takes every read
     auto tally_pass = [&]() -> int {
         SSB_CUDA(ctx, cudaMemsetAsync(err64, 0, ((size_t)n_cov + 1) * sizeof(unsigned long long), s));
         SSB_CUDA(ctx, cudaMemsetAsync(minus, 0, ((size_t)n_cov + 1) * sizeof(unsigned int), s));
-        if (use_list) {
-            if (n_list) SSB_LAUNCH_P(ctx, SSB_K_SPIKE_TALLY, tally_resolve_kernel, grid_for((size_t)n_list, 128), 128, 0, s, TA, exc_list, n_list, keep, kord);
-        } else {
-            KMeta *kmeta = ar.get<KMeta>(K); SPK_CHECK_ARENA(ar);
-            SSB_LAUNCH_P(ctx, SSB_K_SPIKE_TALLY, kmeta_kernel, grid_for(K, 256), 256, 0, s, recs, k_rec, K, kmeta);
-            SSB_LAUNCH_P(ctx, SSB_K_SPIKE_TALLY, tally_fast_kernel, grid_for(K * 32, 128), 128, 0, s, TA, kmeta);
-        }
+        if (use_list && n_list) SSB_LAUNCH_P(ctx, SSB_K_SPIKE_TALLY, tally_resolve_kernel, grid_for((size_t)n_list, 128), 128, 0, s, TA, exc_list, n_list, keep, kord);
         SSB_LAUNCH_P(ctx, SSB_K_SPIKE_TALLY, tally_kernel, grid_for(K, 128), 128, 0, s, TA);
         return SSB_OK;
     };

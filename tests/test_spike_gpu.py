@@ -356,6 +356,21 @@ def test_error_rich_reads_overflow_the_tile_exception_buffer(tmp_path, ctx):
     assert vcf_cmp(want[3], got[3]), "truth.vcf differs: " + first_diff(want[3], got[3])
 
 
+def test_error_rich_reads_overflow_the_exception_list(tmp_path, ctx):
+    """The same error rates over 60 kb: every 32 KiB tile hands over a full 1024-entry buffer, more than the whole exception list
+    holds (n/96 + 65536 entries for n bytes of SAM) once the body passes ~3 MB, so the list overflows and the generic tally takes
+    every read."""
+    prefix = sc.generate("plain", str(tmp_path), contigs="chr19:60000", coverage=40, sub=0.15, q0=0.1, nrate=0.02, spikes=150)
+    n = os.path.getsize(prefix + ".sam")
+    assert (n // 32768) * 1024 > n // 96 + 65536
+    want = sc.run_cli(sc.CHECKER, prefix, str(tmp_path / "ora"), cmdname="stochasticSpike")
+    got = sc.run_cli(sc.PRODUCT, prefix, str(tmp_path / "gpu"))
+    assert want[0] == 0 and got[0] == 0, got[4]
+    assert got[2] == want[2], "SAM differs: " + first_diff(want[2], got[2])
+    assert got[1] == want[1]
+    assert vcf_cmp(want[3], got[3]), "truth.vcf differs: " + first_diff(want[3], got[3])
+
+
 def _with_float_tags(sam: bytes, bad_line=None) -> bytes:
     """Every alignment line gets de:f / B:f fields in the form "%g" prints (what htslib would print back unchanged)."""
     import random

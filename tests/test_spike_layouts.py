@@ -5,7 +5,7 @@ Which code only acts differently when there are many contigs, and where it is ch
 - RNAME / RNEXT lookup (sam_parse.cuh name_lookup): names that are prefixes of one another, HLA names with '*' and ':', RNEXT naming
   a decoy or HLA contig: test_builder_places_the_layout, then every parity test.
 - the reference window staged per tile for its lowest tid (sam_parse.cuh): tiles that span several contigs (the scaffolds),
-  test_builder_places_the_layout; the generic tally against the exception list, test_abi_modes_agree (SSB_NO_EXC_LIST).
+  test_builder_places_the_layout; the exception-list tally against the generic tally of every read, test_abi_modes_agree (SSB_NO_EXC_LIST).
 - packed 32-bit against 8-byte output-order keys (spike_run.cuh): test_key_boundary_bits, then test_abi_modes_agree (SSB_SORT64
   against the packed default on key_boundary) and test_main_matches_checker.
 - (tid, pos) keys over thousands of contigs, covered runs from a contig's first to its last base, targets on contigs without reads,

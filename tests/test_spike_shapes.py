@@ -220,7 +220,7 @@ def _load(prefix):
 
 @pytest.mark.gpu
 def test_chain_modes_agree(tmp_path, ctx, monkeypatch):
-    """The one-warp serial chain, the chunked chain at small geometries, the tally_fast_kernel fallback (no exception list) and the
+    """The one-warp serial chain, the chunked chain at small geometries, the generic tally of every read (no exception list) and the
     8-byte end-order keys: same SAM (the checker's), same per-target results, draw count and SEQ_ERROR records."""
     from stochasticsim_b200 import spike as sp
     prefix, _, _ = _case(tmp_path, "mixed", MIXED_SEED)
